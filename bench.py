@@ -2,6 +2,7 @@
 """bench.py -- path-steps/sec per training iteration of the fused path-space rollout (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c1|c3|c3re|c4|c5]
+                    [--dump-outputs DIR]
 
 Workload (default): BASELINE.json configs[4], the configuration north_star's target is quoted on -- the large-batch
 sweep, LLGC(d=100, off_diag=0, T=1), DenseNet(101 -> 30 -> 30 -> 100) 'inner', K = 2^20 trajectories per GPU,
@@ -19,6 +20,11 @@ Arms
   ours        the CUDA path through pspde.Solver (fails without a GPU: there is no CPU fallback)
   reference   the reference's CPU algorithm (oracle/ref_port.py: PyTorch eager + autograd + CPU randn, the exact
               procedure of solver.py:420-531) on the host cores, on a bounded sample of the same workload
+
+--dump-outputs DIR (ours) writes what the last timed step computed as DIR/<name>.npy: loss (float64), the parameters
+theta after the step's Adam update and their gradient grad (float32), and rank 0's per-path outputs (float32; Y_N, gX,
+X_N, or V0, VE, Y, X_end, t_end for c4) on a fixed, seeded sample of at most 2^16 paths whose indices are path_index
+(float64).  Inputs are seeded, so the same arguments give the same inputs on every run and build.
 """
 import argparse
 import ctypes
@@ -35,6 +41,7 @@ PKG = os.path.join(ROOT, "path-space-pde-solver_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree it runs from (which may be read-only)
 
 import numpy as np  # noqa: E402
 import torch as pt  # noqa: E402
@@ -42,6 +49,8 @@ import torch as pt  # noqa: E402
 METRIC = "path-steps/sec per train iter"
 UNIT = "path-steps/s"
 CPU_SAMPLE_K = 1 << 14          # SURVEY.md section 8(d): K_cpu = min(K, 2^14)
+DUMP_PATHS = 1 << 16            # --dump-outputs: per-path outputs of at most this many paths (seeded sample)
+DUMP_MAX_BYTES = 64 << 20
 
 WORKLOADS = {
     # name: (problem kind, ctor kwargs, net, time_approx, K per GPU, delta_t, loss, detach, lr)
@@ -292,6 +301,27 @@ def timed_steps(rig, S, first, steps):
         ms.append(e0.elapsed_time(e1))
     rig.barrier()
     return rig.max_over_ranks(sum(ms))
+
+
+def dump_outputs(out_dir, whole, per_path):
+    """--dump-outputs: `whole` (name -> tensor or number) as is, `per_path` (name -> tensor with one row per local path)
+    on the paths of a sample that depends only on the number of paths, as out_dir/<name>.npy in float32 / float64."""
+    K = next(iter(per_path.values())).shape[0]
+    rows = np.arange(K) if K <= DUMP_PATHS else np.sort(np.random.default_rng(0).choice(K, DUMP_PATHS, replace=False))
+    arrays = {name: np.asarray(v, dtype=np.float64) for name, v in whole.items() if not pt.is_tensor(v)}
+    arrays.update({name: v.detach().cpu().numpy() for name, v in whole.items() if pt.is_tensor(v)})
+    sel = pt.from_numpy(rows)
+    arrays.update({name: v.detach()[sel.to(v.device)].cpu().numpy() for name, v in per_path.items()})
+    arrays["path_index"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError("--dump-outputs: %s is %s, not float32 / float64" % (name, a.dtype))
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def timed_e2e(rig, S, eng, first, steps):
@@ -610,6 +640,9 @@ def run_ours(args, wl):
     # ---- timed region A: device-timed steps
     total_ms = timed_steps(rig, S, args.warmup, args.steps)
     launches = lib.pspde_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": [S.loss_log[-1]], "theta": S._theta, "grad": S._theta.grad},
+                     {"Y_N": eng.Y_N, "gX": eng.gX, "X_N": eng.X_N})
     ms_per_step = total_ms / args.steps
     value = K_global * N * args.steps / (total_ms * 1e-3)
     # ---- timed region B: end to end through the public API with host inputs
@@ -720,6 +753,9 @@ def run_ours_c4(args, wl):
         step_ms.append(e0.elapsed_time(e1))
     barrier()
     launches = lib.pspde_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": [G.loss_log[-1]], "theta": G._theta, "grad": G._theta.grad},
+                     {"V0": eng.V0, "VE": eng.VE, "Y": eng.Y, "X_end": eng.X_end, "t_end": eng.t_end})
     t = pt.tensor([sum(step_ms)], dtype=pt.float64, device=dev)
     if world > 1:
         td.all_reduce(t, op=td.ReduceOp.MAX)
@@ -834,7 +870,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the c2 / strong / sharding / accuracy blocks")
     ap.add_argument("--accuracy-iters", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
