@@ -60,6 +60,25 @@ def normals(seed, offset, k_global, n, d):
     return z.reshape(k_global.size, nb * 4)[:, :d]
 
 
+def u01(r):
+    """uint32 -> float32 uniform in (0, 1), as in csrc/philox.cuh."""
+    return ((r >> np.uint32(8)).astype(np.float32) + np.float32(0.5)) * np.float32(2.0 ** -24)
+
+
+def ball_and_time(seed, offset, k_offset, K, d, radius, T):
+    """Restatement of diffusion_sample_kernel (csrc/diffusion_kernels.cuh): X_0 uniform in the ball of radius R (the
+    normals of counters (k, 0xFFFFFFFF, jb, offset), normalised, times R u_0^(1/d)) and t_0 = u_1 T in [0, T), where
+    (u_0, u_1) are the first two uniforms of counter (k, 0xFFFFFFFE, 0, offset).  float64 from the float32 draws."""
+    ks = np.arange(k_offset, k_offset + K)
+    z = normals(seed, offset, ks, 0xFFFFFFFF, d).astype(np.float64)
+    ctr = np.zeros((K, 4), np.uint32)
+    ctr[:, 0], ctr[:, 1], ctr[:, 3] = ks, 0xFFFFFFFE, offset & 0xFFFFFFFF
+    key = np.array([seed & 0xFFFFFFFF, (seed >> 32) & 0xFFFFFFFF], dtype=np.uint32)
+    u = u01(philox4x32_10(ctr, key)).astype(np.float64)
+    scale = radius / np.sqrt((z ** 2).sum(1)) * u[:, 0] ** (1.0 / d)
+    return z * scale[:, None], u[:, 1] * T
+
+
 def xi_tensor(seed, offset, k_offset, K, d, N):
     """Reference-layout noise tensor (K, d, N+1); slice 0 is unused by the reference and left zero."""
     xi = np.zeros((K, d, N + 1), np.float32)

@@ -108,6 +108,17 @@ static inline int choose_r(int nng, int T, int rmax) {
   return best;
 }
 
+// Debugging hook PSPDE_MAX_GRID=n: at most n CTAs, so that each CTA loops over more tiles.  make_plan and
+// make_diff_plan apply it last, after their own choice of grid (the attached kernel's two CTAs per SM included) and
+// before the per-CTA workspace sizes (stats, gradient partials, checkpoints), which follow the grid.  A workspace
+// sized with the hook set is too small once it is unset: the launch then fails with -7.
+static inline void apply_max_grid(int& grid) {
+  if (const char* mg = getenv("PSPDE_MAX_GRID")) {
+    const int v = atoi(mg);
+    if (v > 0 && v < grid) grid = v;
+  }
+}
+
 static inline int make_plan(const pspde_cfg* c, bool bwd, bool attached, Plan& pl) {
   int rc = validate(c);
   if (rc) return rc;
@@ -120,10 +131,6 @@ static inline int make_plan(const pspde_cfg* c, bool bwd, bool attached, Plan& p
   const int sms = pspde_sm_count();
   if (sms <= 0) return fail(-10, "no CUDA device");
   pl.grid = pl.n_tiles < sms ? pl.n_tiles : sms;
-  if (const char* mg = getenv("PSPDE_MAX_GRID")) {   // debugging hook: fewer CTAs -> more tiles per CTA
-    const int v = atoi(mg);
-    if (v > 0 && v < pl.grid) pl.grid = v;
-  }
   pl.T = 512; pl.NB = 1;
   if (bwd) {   // one 8x8 weight-gradient block (64 accumulators) per thread
     const int nb = pl.g.n_blocks;
@@ -145,6 +152,7 @@ static inline int make_plan(const pspde_cfg* c, bool bwd, bool attached, Plan& p
     const char* e = getenv("PSPDE_ATT_CTAS");
     if (!(e && e[0] == '1')) { pl.ctas_per_sm = 2; pl.grid = pl.n_tiles < 2 * sms ? pl.n_tiles : 2 * sms; }
   }
+  apply_max_grid(pl.grid);
   pl.stats_bytes = align256((size_t)pl.grid * 4 * sizeof(double));
   pl.grad_bytes = bwd ? align256((size_t)pl.grid * pl.n_img_total * sizeof(float)) : 0;
   return 0;

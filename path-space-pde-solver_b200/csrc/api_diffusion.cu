@@ -57,6 +57,7 @@ int make_diff_plan(const pspde_cfg* c, float T_end, DiffPlan& pl, const pspde_el
   pl.grid = pl.n_tiles < sms ? pl.n_tiles : sms;
   pl.smem_bytes = (size_t)diff_smem_layout(pl.g, kPD).total * sizeof(float);
   if (pl.smem_bytes > kMaxSmem) return fail(-6, "network + tile need %zu B of shared memory (> %zu)", pl.smem_bytes, kMaxSmem);
+  apply_max_grid(pl.grid);
   pl.stats_bytes = align256((size_t)pl.grid * 4 * sizeof(double));
   pl.wpack_bytes = align256((size_t)pl.g.w_floats * sizeof(float));
   pl.grad_bytes = align256((size_t)pl.grid * dw_partial_floats(pl.g) * sizeof(float));

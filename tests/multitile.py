@@ -1,0 +1,371 @@
+"""Cases shared by test_emu_multitile.py (host emulator) and test_gpu_multitile.py (sm_100a build): the attached adjoint
+kernel and the diffusion / elliptic kernels with several tiles per CTA, against the fp64 oracle (oracle/manual.py).
+
+A persistent CTA loops `for (tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)`: per-tile state must be reset and
+the per-CTA gradient partials must collect every tile exactly once.  Each case is run by the test files at a K that
+gives at least two tiles per CTA at the natural grid, and again with PSPDE_MAX_GRID for many tiles per CTA.  The
+last tile is always ragged.  The increments are the kernels' own Philox draws, read back with pspde_philox_dump.
+
+`Abi` drives the C ABI with numpy buffers (emulator) or CUDA tensors (device), so both files run the same code."""
+import ctypes
+
+import numpy as np
+
+import emu_harness as H
+from conftest import relerr
+from oracle import manual as man
+from pspde import _lib as L
+
+TOL_PATH, TOL_END, TOL_GRAD, TOL_BLOCK = 1e-5, 1e-6, 2e-5, 5e-5
+P_HJB, P_DIFF = 64, 32          # paths per tile of the rollout / attached kernels and of the diffusion kernel
+
+
+class Abi:
+    """The library's entry points on host (device=None: numpy, emulator build) or device (torch CUDA tensors) buffers;
+    inputs and outputs are numpy arrays either way."""
+
+    def __init__(self, lib, device=None):
+        self.lib, self.device = lib, device
+        if device is not None:
+            import torch
+            self.pt = torch
+
+    def dev(self, a, dtype=np.float32):
+        if a is None:
+            return None
+        a = np.ascontiguousarray(a, dtype)
+        return a if self.device is None else self.pt.from_numpy(a).to(self.device)
+
+    def zeros(self, shape, dtype=np.float32):
+        a = np.zeros(shape, dtype)
+        return a if self.device is None else self.pt.from_numpy(a).to(self.device)
+
+    def host(self, a):
+        return a if self.device is None else a.cpu().numpy()
+
+    def p(self, a):
+        """Raw pointer; a device tensor passed here must stay referenced until the call returns (the caching allocator
+        reuses a freed block for the next upload before the kernel runs)."""
+        if a is None:
+            return None
+        return a.ctypes.data_as(ctypes.c_void_p) if self.device is None else ctypes.c_void_p(a.data_ptr())
+
+    def ws(self, nbytes):
+        assert nbytes > 0, self.lib.pspde_last_error()
+        return self.zeros(nbytes // 8 + 1, np.float64)
+
+    def nbytes(self, a):
+        return a.nbytes if self.device is None else a.numel() * a.element_size()
+
+    def _out(self, names):
+        return {k: self.zeros(s, np.float64 if k == "stats" else np.float32) for k, s in names.items()}
+
+    def _host_all(self, o):
+        return {k: self.host(v) for k, v in o.items()}
+
+    # -- HJB rollout
+    def philox_dump(self, cfg):
+        """(N, K, d) float32: the increments the kernels draw for cfg."""
+        out = self.zeros((cfg.N, cfg.K_local, cfg.d))
+        L.check(self.lib, self.lib.pspde_philox_dump(ctypes.byref(cfg), self.p(out), None))
+        return self.host(out)
+
+    def fwd(self, cfg, theta, pack, x0):
+        K, d = cfg.K_local, cfg.d
+        ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
+        o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4))
+        ins = [self.dev(a) for a in (theta, pack, x0)]
+        rc = self.lib.pspde_rollout_fwd(ctypes.byref(cfg), *[self.p(a) for a in ins], None, None, self.p(o["X"]),
+                                        self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]), self.p(o["stats"]), self.p(ws),
+                                        self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self._host_all(o)
+
+    def attached(self, cfg, theta, pack, x0, w, wY=None, wZ=None, wG=None):
+        K, d = cfg.K_local, cfg.d
+        ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
+        o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4, grad=self.lib.pspde_theta_size(ctypes.byref(cfg))))
+        keep = [self.dev(a) for a in (theta, pack, x0, wY, wZ, wG)]
+        rc = self.lib.pspde_rollout_attached(ctypes.byref(cfg), *[self.p(a) for a in keep[:3]], None, None,
+                                             ctypes.c_float(w), *[self.p(a) for a in keep[3:]], self.p(o["X"]),
+                                             self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]), self.p(o["stats"]),
+                                             self.p(o["grad"]), self.p(ws), self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self._host_all(o)
+
+    # -- diffusion / elliptic
+    def diff_fwd(self, cfg, T, theta, pack, X0, t0, xis, ell=None):
+        K, d = cfg.K_local, cfg.d
+        o = self._out(dict(V0=K, VE=K, Y=K, X=(K, d), t=K, VL2=K, stats=4))
+        ins = [self.dev(a) for a in (theta, pack, X0, t0, xis)]
+        if ell is None:
+            ws = self.ws(self.lib.pspde_diffusion_workspace_bytes(ctypes.byref(cfg), ctypes.c_float(T)))
+            rc = self.lib.pspde_diffusion_fwd(ctypes.byref(cfg), ctypes.c_float(T), *[self.p(a) for a in ins],
+                                              self.p(o["V0"]), self.p(o["VE"]), self.p(o["Y"]), self.p(o["X"]),
+                                              self.p(o["t"]), self.p(o["stats"]), self.p(ws), self.nbytes(ws), None)
+        else:
+            ws = self.ws(self.lib.pspde_elliptic_workspace_bytes(ctypes.byref(cfg), ctypes.byref(ell)))
+            rc = self.lib.pspde_elliptic_fwd(ctypes.byref(cfg), ctypes.byref(ell), self.p(ins[0]), self.p(ins[1]),
+                                             self.p(ins[2]), self.p(ins[4]), self.p(o["V0"]), self.p(o["VE"]),
+                                             self.p(o["Y"]), self.p(o["X"]), self.p(o["VL2"]), self.p(o["stats"]),
+                                             self.p(ws), self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self._host_all(o)
+
+    def diff_bwd(self, cfg, T, theta, pack, X0, t0, xis, c0, cE, cD, ell=None):
+        grad = self.zeros(self.lib.pspde_theta_size(ctypes.byref(cfg)))
+        ins = [self.dev(a) for a in (theta, pack, X0, t0, xis, c0, cE, cD)]
+        if ell is None:
+            ws = self.ws(self.lib.pspde_diffusion_workspace_bytes(ctypes.byref(cfg), ctypes.c_float(T)))
+            rc = self.lib.pspde_diffusion_bwd(ctypes.byref(cfg), ctypes.c_float(T), *[self.p(a) for a in ins],
+                                              self.p(grad), self.p(ws), self.nbytes(ws), None)
+        else:
+            ws = self.ws(self.lib.pspde_elliptic_workspace_bytes(ctypes.byref(cfg), ctypes.byref(ell)))
+            ins = ins[:3] + ins[4:]
+            rc = self.lib.pspde_elliptic_bwd(ctypes.byref(cfg), ctypes.byref(ell), *[self.p(a) for a in ins],
+                                             self.p(grad), self.p(ws), self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self.host(grad)
+
+    def sample(self, cfg, radius, T):
+        X0, t0 = self.zeros((cfg.K_local, cfg.d)), self.zeros(cfg.K_local)
+        L.check(self.lib, self.lib.pspde_diffusion_sample(ctypes.byref(cfg), ctypes.c_float(radius), ctypes.c_float(T),
+                                                          self.p(X0), self.p(t0), None))
+        return self.host(X0), self.host(t0)
+
+
+# ------------------------------------------------------------------------------------------------------------ helpers
+def grad_blocks(kind, dims, n_sets=1):
+    """Slices of theta, one per (parameter set, layer): W_l and b_l of that layer."""
+    out, off = [], 0
+    for _ in range(n_sets):
+        for i in range(len(dims) - 1):
+            fan_in = sum(dims[:i + 1]) if kind == "densenet" else dims[i]
+            n = (fan_in + 1) * dims[i + 1]
+            out.append(slice(off, off + n))
+            off += n
+    return out
+
+
+def n_grad_blocks(kind, dims):
+    """The attached / backward kernels' count of 8x8 weight-gradient blocks (build_geom, csrc/pspde_geom.h): more than
+    224 selects the 512-thread build."""
+    c4 = lambda x: (x + 3) & ~3
+    L_ = len(dims) - 1
+    seg = [c4(dims[s] + (1 if (kind == "mlp_tanh" or s == 0) else 0)) for s in range(L_)]
+    blk = 0
+    for l in range(L_):
+        Kp = sum(seg[:l + 1]) if kind == "densenet" else seg[l]
+        nkg, nng = Kp // 4, c4(dims[l + 1]) // 4
+        blk += ((nkg + 1) // 2) * ((nng + 1) // 2)
+    return blk
+
+
+def check_grad(grad, ref, blocks, what=""):
+    assert np.isfinite(grad).all(), what
+    e = relerr(grad, ref)
+    assert e < TOL_GRAD, (what, e)
+    for i, s in enumerate(blocks):        # a flush into the wrong slice shows up as one bad block
+        assert relerr(grad[s], ref[s]) < TOL_BLOCK, (what, "block", i, relerr(grad[s], ref[s]))
+
+
+def tiles_per_cta(K, P, grid):
+    n_tiles = (K + P - 1) // P
+    return n_tiles / min(n_tiles, grid)
+
+
+# ------------------------------------------------------------------------------------------------ attached kernel
+def hjb_problem(kind, d, off_diag=0.0, seed=0):
+    """(man.Problem, (problem_id, flags, pack), x0) for 'lqgc', 'llgc' (optionally with dense A / B) and 'dwm' (C3's
+    DoubleWell_multidim: d_1 = 15, kappa = 5, eta = 3)."""
+    if kind == "dwm":
+        pkw = dict(d_1=15, d_2=d - 15, eta=3.0, kappa=5.0)
+        eta = np.array([3.0] * 15 + [1.0] * (d - 15))
+        kap = np.array([5.0] * 15 + [1.0] * (d - 15))
+        return man.Problem("dwm", d, eta_=eta, kappa_=kap), H.problem_pack("dwm", d, pkw), -np.ones(d, np.float32)
+    A = B = None
+    if off_diag:
+        rng = np.random.default_rng(seed)
+        A = (-np.eye(d) + off_diag * rng.standard_normal((d, d))).astype(np.float32)
+        B = (np.eye(d) + off_diag * rng.standard_normal((d, d))).astype(np.float32)
+    pk = H.problem_pack(kind, d, {}, A, B)
+    mp = man.Problem(kind, d, A=None if A is None else A.astype(np.float64), B=None if B is None else B.astype(np.float64))
+    return mp, pk, np.zeros(d, np.float32)
+
+
+def attached_case(abi, kind, d, net, K, N, dt, loss, off_diag=0.0, outer=False, inert=False, seed=5, theta=None):
+    """The attached kernel against the fp64 discrete adjoint: relative entropy in one launch (man.grad_mode_b) or a
+    general loss through the forward launch -> per-path cotangents -> adjoint launch (man.grad_attached).  inert: every
+    7th path gets exactly zero cotangents (the oracle gets the same zeros)."""
+    mp, (pid, flags, pack), x0 = hjb_problem(kind, d, off_diag, seed)
+    dims = [d if outer else d + 1, 30, 30, d]
+    n_sets = N if outer else 1
+    tm = L.TIME_NONE if outer else L.TIME_FIRST
+    net_id = L.NET_DENSENET if net == "densenet" else L.NET_MLP_TANH
+    cfg = L.make_cfg(K, d, N, np.float32(dt), pid, net_id, dims, tm, adaptive=True, problem_flags=flags,
+                     noise_mode=L.NOISE_PHILOX, seed=seed, offset=3, n_sets=N if outer else 0)
+    n_theta = abi.lib.pspde_theta_size(ctypes.byref(cfg))
+    assert n_theta > 0, abi.lib.pspde_last_error()
+    if theta is None:
+        theta = (0.1 * np.random.default_rng(seed).standard_normal(n_theta)).astype(np.float32)
+    nth = n_theta // n_sets
+    th64 = theta.astype(np.float64)
+    nets = [man.Net(net, dims, th64[s * nth:(s + 1) * nth]) for s in range(n_sets)]
+    xi = np.zeros((K, d, N + 1))
+    xi[:, :, 1:] = abi.philox_dump(cfg).transpose(1, 2, 0)
+    mode = "none" if outer else "first"
+    if loss == "relative_entropy":
+        o = abi.attached(cfg, theta, pack, x0, 1.0 / K)
+        gm, ro = man.grad_mode_b(mp, nets[0], xi, dt, N, x0.astype(np.float64), mode)
+    else:
+        f = abi.fwd(cfg, theta, pack, x0)
+        _, wY, wZ, wG = man.loss_cotangents_full(loss, f["Y"].astype(np.float64), f["gX"].astype(np.float64),
+                                                 f["Zsum"].astype(np.float64), True)
+        wY, wZ, wG = (np.asarray(w, np.float32) for w in (wY, wZ, wG))
+        if inert:
+            for w in (wY, wZ, wG):
+                w[::7] = 0.0
+        o = abi.attached(cfg, theta, pack, x0, 0.0, wY, wZ, wG)
+        gm, ro = man.grad_attached(mp, nets if outer else nets[0], xi, dt, N, x0.astype(np.float64),
+                                   wY.astype(np.float64), wZ.astype(np.float64), wG.astype(np.float64), mode)
+        for k in ("X", "Y", "Zsum", "gX"):           # the forward launch that produced the cotangents
+            assert relerr(f[k], ro[k]) < TOL_PATH, ("forward launch", k, relerr(f[k], ro[k]))
+    for k in ("X", "Y", "Zsum", "gX"):
+        assert relerr(o[k], ro[k]) < TOL_PATH, ("attached launch", k, relerr(o[k], ro[k]))
+    v = o["Zsum"].astype(np.float64) + o["gX"]
+    assert o["stats"][3] == 0
+    np.testing.assert_allclose(o["stats"][2], v.sum(), rtol=1e-10)
+    check_grad(o["grad"], gm, grad_blocks(net, dims, n_sets), "%s d=%d %s" % (kind, d, loss))
+
+
+# ------------------------------------------------------------------------------------------------ diffusion kernels
+def _theta(dims, seed, scale=0.3):
+    n = sum((sum(dims[:i + 1]) + 1) * dims[i + 1] for i in range(len(dims) - 1))
+    return (scale * np.random.default_rng(seed).standard_normal(n) / np.sqrt(max(dims))).astype(np.float32)
+
+
+def _ball(rng, K, d, r_lo=0.0, r_hi=1.0):
+    z = rng.standard_normal((K, d))
+    r = r_lo + (r_hi - r_lo) * rng.uniform(0, 1, (K, 1)) ** (1.0 / d)
+    return (z / np.linalg.norm(z, axis=1, keepdims=True) * r).astype(np.float32)
+
+
+def _chunked(fn, K, chunk):
+    """Run the oracle over path chunks (one tape per step per chunk bounds its memory); the gradient is a per-path sum,
+    the chunk's loss weight alpha_0 = K_chunk / K keeps w = 2 r / K."""
+    parts = [fn(lo, min(K, lo + chunk), (min(K, lo + chunk) - lo) / K) for lo in range(0, K, chunk)]
+    out = {k: np.concatenate([p[k] for p in parts]) for k in parts[0] if k not in ("grad", "K_count", "loss", "loss_boundary")}
+    out["grad"] = sum(p["grad"] for p in parts)
+    out["K_count"] = sum(p["K_count"] for p in parts)
+    return out
+
+
+_ORACLE = {}
+
+
+def diffusion_case(abi, kind, d, arch, K, N, dt, noise, seed=7, chunk=1024):
+    """GeneralSolver's kernels (heat: h = 0; allencahn: h = y - y^3, which adds the backward's V(X_n) pass) with t_0 in
+    [0.9, 1): every tile mixes moving and stopped paths.  noise 'inject' feeds the Philox dump back as injected draws."""
+    T = 1.0
+    dims = [d + 1] + list(arch) + [1]
+    theta = _theta(dims, seed)
+    rng = np.random.default_rng(seed)
+    X0 = _ball(rng, K, d)
+    t0 = rng.uniform(0.9, 1.0, K).astype(np.float32)
+    pid = L.PROBLEM_HEAT if kind == "heat" else L.PROBLEM_ALLEN_CAHN
+    cfg = H.diffusion_cfg(K, d, N, dt, arch, noise=L.NOISE_PHILOX, seed=seed, offset=2, problem_id=pid)
+    xs = abi.philox_dump(cfg)
+    if noise == "inject":
+        cfg = H.diffusion_cfg(K, d, N, dt, arch, noise=L.NOISE_INJECT, seed=seed, offset=2, problem_id=pid)
+    pack = H.heat_pack(d)
+    xin = xs if noise == "inject" else None
+    f = abi.diff_fwd(cfg, T, theta, pack, X0, t0, xin)
+    r = f["VE"].astype(np.float64) - f["Y"]
+    w = 2 * r / K
+    grad = abi.diff_bwd(cfg, T, theta, pack, X0, t0, xin, -w, w, -w)
+    key = ("diff", kind, d, tuple(arch), K, N, dt, seed, xs.tobytes().__hash__())
+    if key not in _ORACLE:
+        net = man.Net("densenet", dims, theta.astype(np.float64))
+        pde = None if kind == "heat" else man.ALLEN_CAHN
+        X64, t64, x64 = X0.astype(np.float64), t0.astype(np.float64), xs.astype(np.float64)
+
+        def part(lo, hi, a0):
+            m = man.diffusion(man.Problem("heat", d), net, X64[lo:hi], t64[lo:hi], x64[:, lo:hi], dt, N, 1,
+                              alpha=(a0, 0.0, 0.0), T=T, pde=pde)
+            m["VE"] = net.forward(np.concatenate([m["X"], m["t"][:, None]], 1))[0][:, 0]
+            m["V0"] = net.forward(np.concatenate([X64[lo:hi], t64[lo:hi, None]], 1))[0][:, 0]
+            return m
+        _ORACLE[key] = _chunked(part, K, chunk)
+    m = _ORACLE[key]
+    assert 0 < m["K_count"] < K * N and int(f["stats"][1]) == m["K_count"]
+    assert relerr(f["X"], m["X"]) < TOL_END and relerr(f["t"], m["t"]) < TOL_END
+    for k in ("Y", "VE", "V0"):
+        assert relerr(f[k], m[k]) < TOL_PATH, (k, relerr(f[k], m[k]))
+    assert f["stats"][3] == 0
+    np.testing.assert_allclose(f["stats"][[0, 2]], [(r * r).sum(), r.sum()], rtol=1e-9)
+    check_grad(grad, m["grad"], grad_blocks("densenet", dims), "diffusion %s %s" % (kind, noise))
+
+
+def elliptic_case(abi, kind, d, arch, K, N, dt, seed=9, chunk=2048):
+    """EllipticSolver's kernels on the unit ball ('sphere': h = expball_sin), a one-sided box ('box': h =
+    exp-nonlinear, alpha = 1/2) and the committor annulus 1 < |x| < 2 ('committor': h = 0, sigma = I)."""
+    dims = [d] + list(arch) + [1]
+    theta = _theta(dims, seed)
+    rng = np.random.default_rng(seed)
+    pack = H.heat_pack(d)
+    if kind == "sphere":
+        ell, mp, X0 = H.elliptic_spec("expball_sin"), man.EllipticProblem("expball_sin", d), _ball(rng, K, d)
+    elif kind == "box":
+        ell = L.make_elliptic(L.DOMAIN_BOX, x_l=-1.0, x_r=1.0, one_boundary=True, h_id=L.H_EXP_NONLINEAR,
+                              h_param=(0.5, 0, 0))
+        mp = man.EllipticProblem("expball", d, alpha=0.5)
+        mp.boundary, mp.one_boundary, mp.X_l, mp.X_r = "square", True, -1.0, 1.0
+        X0 = rng.uniform(-1, 1, (K, d)).astype(np.float32)
+    else:
+        ell, mp, X0 = H.elliptic_spec("committor"), man.EllipticProblem("committor", d), _ball(rng, K, d, 1.02, 1.98)
+        pack[d:2 * d] = 1.0
+    cfg = H.elliptic_cfg(K, d, N, dt, arch, noise=L.NOISE_PHILOX, seed=seed, offset=1, k_offset=3)
+    xs = abi.philox_dump(cfg)
+    f = abi.diff_fwd(cfg, 1.0, theta, pack, X0, None, None, ell=ell)
+    r = f["VE"].astype(np.float64) - f["Y"]
+    w = 2 * r / K
+    grad = abi.diff_bwd(cfg, 1.0, theta, pack, X0, None, None, -w, w, -w, ell=ell)
+    key = ("ell", kind, d, tuple(arch), K, N, dt, seed, xs.tobytes().__hash__())
+    if key not in _ORACLE:
+        net = man.Net("densenet", dims, theta.astype(np.float64))
+        X64, x64 = X0.astype(np.float64), xs.astype(np.float64)
+
+        def part(lo, hi, a0):
+            m = man.elliptic(mp, net, X64[lo:lo + 1], X64[lo:hi], x64[:, lo:hi], dt, N, alpha=(a0, 0.0))
+            m["VE"] = m["r"] + m["Y"]
+            return m
+        _ORACLE[key] = _chunked(part, K, chunk)
+    m = _ORACLE[key]
+    assert 0 < m["K_count"] < K * N and int(f["stats"][1]) == m["K_count"]
+    assert relerr(f["X"], m["X"]) < TOL_END
+    for k in ("Y", "VE"):
+        assert relerr(f[k], m[k]) < TOL_PATH, (k, relerr(f[k], m[k]))
+    assert relerr(f["VL2"], m["V_L2"]) < (1e-4 if kind == "committor" else TOL_PATH), relerr(f["VL2"], m["V_L2"])
+    assert f["stats"][3] == 0
+    np.testing.assert_allclose(f["stats"][[0, 2]], [(r * r).sum(), r.sum()], rtol=1e-9)
+    check_grad(grad, m["grad"], grad_blocks("densenet", dims), "elliptic %s" % kind)
+
+
+# ------------------------------------------------------------------------------------------------ start points
+def sample_case(abi, K, d, k_offset, seed=11, offset=4, radius=1.5, T=1.0):
+    """diffusion_sample_kernel against its restatement (oracle/philox.py::ball_and_time)."""
+    from oracle import philox as ph
+    cfg = H.diffusion_cfg(K, d, 1, 0.01, (8,), noise=L.NOISE_PHILOX, k_offset=k_offset, seed=seed, offset=offset)
+    X0, t0 = abi.sample(cfg, radius, T)
+    Xr, tr = ph.ball_and_time(seed, offset, k_offset, K, d, radius, T)
+    assert relerr(X0, Xr) < TOL_PATH and relerr(t0, tr) < TOL_PATH
+    assert np.abs(np.linalg.norm(X0, axis=1) - np.linalg.norm(Xr, axis=1)).max() < TOL_PATH * radius
+    return X0, t0
+
+
+def sample_uniformity(X0, t0, radius, T):
+    """(|X_0| / R)^d and t_0 / T are U(0, 1) if X_0 is uniform in the ball and t_0 uniform in [0, T): KS p-values."""
+    from scipy import stats
+    d = X0.shape[1]
+    rad = (np.linalg.norm(X0.astype(np.float64), axis=1) / radius) ** d
+    return stats.kstest(rad, "uniform").pvalue, stats.kstest(t0.astype(np.float64) / T, "uniform").pvalue
