@@ -110,8 +110,9 @@ static inline int choose_r(int nng, int T, int rmax) {
 
 // Debugging hook PSPDE_MAX_GRID=n: at most n CTAs, so that each CTA loops over more tiles.  make_plan and
 // make_diff_plan apply it last, after their own choice of grid (the attached kernel's two CTAs per SM included) and
-// before the per-CTA workspace sizes (stats, gradient partials, checkpoints), which follow the grid.  A workspace
-// sized with the hook set is too small once it is unset: the launch then fails with -7.
+// before the per-CTA workspace sizes (stats, gradient partials, checkpoints), which follow the grid.  The tensor-core
+// launches of api_core.cu (forward, checkpoint rollout, gradient kernels) apply it to their own grids the same way.  A
+// workspace sized with the hook set is too small once it is unset: the launch then fails with -7.
 static inline void apply_max_grid(int& grid) {
   if (const char* mg = getenv("PSPDE_MAX_GRID")) {
     const int v = atoi(mg);

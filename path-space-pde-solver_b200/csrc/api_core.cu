@@ -78,9 +78,10 @@ static int ckpt_cols_of(const TcGeom& tg, int ckpt_zeta) { return ckpt_zeta ? tc
 
 // Forward rollout launch: the tensor-core kernel (rollout_tc_kernels.cuh) for the shape class it covers, else the
 // FP32-FMA kernel.  PSPDE_FWD_PATH=simt forces the FMA kernel (A/B tests); PSPDE_FWD_PATH=tc makes an ineligible
-// configuration an error.  *grid_out = number of CTAs launched (rows of stats_partial that were written).
+// configuration an error.  *grid_out = number of CTAs launched (rows of stats_partial that were written); stats_room = bytes
+// the caller's workspace holds for those rows.
 static int launch_forward(const pspde_cfg* cfg, const Plan& pl, RolloutParams& p, bool tc_allowed, void* stream, int* grid_out,
-                          int keep_tiles = 0) {
+                          size_t stats_room, int keep_tiles = 0) {
   const bool keep_ckpt = keep_tiles > 0;
 #if !defined(PSPDE_EMULATE)
   TcGeom tg;
@@ -90,7 +91,12 @@ static int launch_forward(const pspde_cfg* cfg, const Plan& pl, RolloutParams& p
   if (eligible && !(path && !strcmp(path, "simt"))) {
     const int n_tiles = (cfg->K_local + kTcP - 1) / kTcP;
     const int sms = pspde_sm_count();
-    const int grid = n_tiles < sms ? n_tiles : sms;
+    int grid = n_tiles < sms ? n_tiles : sms;
+    apply_max_grid(grid);
+    // every CTA writes 4 stats doubles at stats_partial[4 blockIdx.x]: checked against the caller's workspace (pl.stats_bytes
+    // counts pl.grid CTAs of 64-path tiles, not this grid)
+    if ((size_t)grid * 4 * sizeof(double) > stats_room)
+      return fail(-7, "workspace too small for the forward's statistics (%zu < %zu)", stats_room, (size_t)grid * 4 * sizeof(double));
     p.n_tiles = n_tiles;
     if (keep_ckpt) { p.ckpt_zeta = zeta_in_ckpt(cfg, nullptr); p.ckpt_cols = ckpt_cols_of(tg, p.ckpt_zeta); p.ckpt_s0 = tg.s0;
                      p.tile0 = 0; p.ckpt_unit = 1; p.ckpt_tiles = keep_tiles; }
@@ -231,6 +237,9 @@ static bool ckpt_plan(const pspde_cfg* cfg, const Plan& pl, TcGeom& tg, CkptPlan
   cp.s0 = tg.s0;
   const long long n_ts = (long long)cp.wave * cfg->N;
   cp.grid_b = n_ts < sms ? (int)n_ts : sms;
+  // PSPDE_MAX_GRID caps the gradient CTAs but not the wave (still per_sm x SMs tiles): each CTA then runs more stages per
+  // launch and flushes its accumulators many times, as at C5, at a K small enough for the fp64 oracle
+  apply_max_grid(cp.grid_b);
   cp.ckpt_bytes = align256((size_t)cp.wave * cfg->N * cp.cols * kTcP * 4);
   cp.grad_bytes = align256((size_t)cp.grid_b * grad_part_floats(cfg, pl, tg.s0) * sizeof(float));
   return true;
@@ -269,7 +278,9 @@ static int run_waves(const pspde_cfg* cfg, const Plan& pl, RolloutParams& p, con
   for (int t0 = t_begin; t0 < cp.n_tiles128; t0 += cp.wave) {
     const int nt = cp.n_tiles128 - t0 < cp.wave ? cp.n_tiles128 - t0 : cp.wave;
     p.tile0 = t0; p.n_tiles = nt; p.ckpt_tiles = nt;
-    const cudaError_t ce = tc_launch_t<true>(p, tg, nt < sms ? nt : sms, (cudaStream_t)stream);
+    int grid_f = nt < sms ? nt : sms;
+    apply_max_grid(grid_f);
+    const cudaError_t ce = tc_launch_t<true>(p, tg, grid_f, (cudaStream_t)stream);
     g_launches++;
     if (ce != cudaSuccess) return fail(-12, "tensor-core checkpoint rollout launch failed: %s", cudaGetErrorString(ce));
     const long long n_ts = (long long)nt * cfg->N;
@@ -408,7 +419,7 @@ int pspde_rollout_fwd_ckpt(const pspde_cfg* cfg, const float* theta, const float
   p.stats_partial = reinterpret_cast<double*>(workspace);
   p.ckpt = reinterpret_cast<float*>(ckpt);
   int grid = pl.grid;
-  rc = launch_forward(cfg, pl, p, true, stream, &grid, keep_tiles);
+  rc = launch_forward(cfg, pl, p, true, stream, &grid, workspace_bytes, keep_tiles);
   if (rc) return rc;
   if (stats) {
     PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, grid, stats);
@@ -479,7 +490,8 @@ int pspde_grad_from_ckpt(const pspde_cfg* cfg, const float* theta, const float* 
     return fail(-6, "configuration is outside the checkpointed backward's shape class");
   const int sms = pspde_sm_count();
   const long long n_ts = (long long)n_slots * cfg->N;
-  const int grid = n_ts < sms ? (int)n_ts : sms;
+  int grid = n_ts < sms ? (int)n_ts : sms;
+  apply_max_grid(grid);
   const size_t gbytes = align256((size_t)grid * grad_part_floats(cfg, pl, s0) * sizeof(float));
   if (!workspace || workspace_bytes < pl.stats_bytes + gbytes) return fail(-7, "workspace too small (%zu < %zu)", workspace_bytes, pl.stats_bytes + gbytes);
   if (misaligned16(workspace)) return fail(-7, "workspace must be 16-byte aligned");
@@ -514,6 +526,7 @@ int pspde_grad_from_fwd_ckpt(const pspde_cfg* cfg, const float* theta, const flo
   const int n_keep = (int)((ckpt_bytes < need ? ckpt_bytes : need) / tb);       // tiles whose rows the forward kept
   const long long n_ts = (long long)n_keep * cfg->N;
   int grid = n_ts < sms ? (int)n_ts : sms;
+  apply_max_grid(grid);
   size_t gbytes = align256((size_t)grid * grad_part_floats(cfg, pl, tg.s0) * sizeof(float));
   size_t ws_need = pl.stats_bytes + gbytes;
   CkptPlan cp;
@@ -620,7 +633,7 @@ int pspde_importance_sampling(const pspde_cfg* cfg, const float* theta, const fl
   p.t_index = t_index; p.dt_net = dt_net;
   p.stats_partial = reinterpret_cast<double*>(workspace);
   int grid = pl.grid;
-  return launch_forward(cfg, pl, p, true, stream, &grid);
+  return launch_forward(cfg, pl, p, true, stream, &grid, workspace_bytes);
 }
 
 int pspde_philox_dump(const pspde_cfg* cfg, float* xi_out, void* stream) {

@@ -1,5 +1,6 @@
 """Cases shared by test_emu_multitile.py (host emulator) and test_gpu_multitile.py (sm_100a build): the attached adjoint
 kernel and the diffusion / elliptic kernels with several tiles per CTA, against the fp64 oracle (oracle/manual.py).
+TcCase and check_tc_forward serve test_gpu_tc_multitile.py (tensor-core kernels, device only).
 
 A persistent CTA loops `for (tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)`: per-tile state must be reset and
 the per-CTA gradient partials must collect every tile exactly once.  Each case is run by the test files at a K that
@@ -132,6 +133,56 @@ class Abi:
         L.check(self.lib, self.lib.pspde_diffusion_sample(ctypes.byref(cfg), ctypes.c_float(radius), ctypes.c_float(T),
                                                           self.p(X0), self.p(t0), None))
         return self.host(X0), self.host(t0)
+
+    # -- tensor-core rollout and gradient kernels (device only: tcgen05 has no host emulation)
+    def fwd_ckpt(self, cfg, theta, pack, x0, xi=None, table=None, ckpt_bytes=0):
+        """pspde_rollout_fwd_ckpt: the forward, with the u_L2 diagnostic (mode 1, linear table) if `table` is given and
+        keeping the operand rows of its first tiles in a buffer of ckpt_bytes if that is > 0.  Returns (outputs,
+        device checkpoint buffer or None, launches it took)."""
+        K, d = cfg.K_local, cfg.d
+        ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
+        o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4, uL2=K))
+        ins = [self.dev(a) for a in (theta, pack, x0, xi, table)]
+        diag = None
+        if table is not None:
+            diag = L.pspde_udiag(mode=1, nx1=0, d1=0, xb=0.0, dx=0.0, table=ins[4].data_ptr(), uL2=o["uL2"].data_ptr(),
+                                 quirk_path=-1)
+        ck = self.zeros(ckpt_bytes // 4) if ckpt_bytes else None
+        n0 = self.lib.pspde_launch_count()
+        rc = self.lib.pspde_rollout_fwd_ckpt(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], None, self.xi_ptr(ins[3]),
+                                             self.p(o["X"]), self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]),
+                                             self.p(o["stats"]), None if diag is None else ctypes.byref(diag), self.p(ck),
+                                             ckpt_bytes, self.p(ws), self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self._host_all(o), ck, self.lib.pspde_launch_count() - n0
+
+    def xi_ptr(self, xi):
+        """Injected increments in the reference layout (K, d, N + 1): slice n + 1 drives step n."""
+        return None if xi is None else ctypes.c_void_p(xi.data_ptr() + 4 * xi.stride(2))
+
+    def bwd_detached(self, cfg, theta, pack, x0, wY, wZ=None, xi=None):
+        """pspde_rollout_bwd_detached: (gradient, launches it took)."""
+        grad = self.zeros(self.lib.pspde_theta_size(ctypes.byref(cfg)))
+        ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
+        ins = [self.dev(a) for a in (theta, pack, x0, xi, wY, wZ)]
+        n0 = self.lib.pspde_launch_count()
+        rc = self.lib.pspde_rollout_bwd_detached(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], self.xi_ptr(ins[3]),
+                                                 self.p(ins[4]), self.p(ins[5]), self.p(grad), self.p(ws), self.nbytes(ws),
+                                                 None)
+        L.check(self.lib, rc)
+        return self.host(grad), self.lib.pspde_launch_count() - n0
+
+    def grad_from_fwd_ckpt(self, cfg, theta, pack, x0, ck, wY, xi=None):
+        """pspde_grad_from_fwd_ckpt on the rows a fwd_ckpt call kept: (gradient, launches it took)."""
+        grad = self.zeros(self.lib.pspde_theta_size(ctypes.byref(cfg)))
+        ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
+        ins = [self.dev(a) for a in (theta, pack, x0, xi, wY)]
+        n0 = self.lib.pspde_launch_count()
+        rc = self.lib.pspde_grad_from_fwd_ckpt(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], self.xi_ptr(ins[3]),
+                                               self.p(ck), self.nbytes(ck), self.p(ins[4]), self.p(grad), self.p(ws),
+                                               self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self.host(grad), self.lib.pspde_launch_count() - n0
 
 
 # ------------------------------------------------------------------------------------------------------------ helpers
@@ -369,3 +420,101 @@ def sample_uniformity(X0, t0, radius, T):
     d = X0.shape[1]
     rad = (np.linalg.norm(X0.astype(np.float64), axis=1) / radius) ** d
     return stats.kstest(rad, "uniform").pvalue, stats.kstest(t0.astype(np.float64) / T, "uniform").pvalue
+
+
+# ------------------------------------------------------------------------------------------ tensor-core rollout / gradient
+P_TC = 128                      # paths per tile of rollout_tc_fwd_kernel (tensor-memory lanes)
+
+# Shapes of the tensor-core kernels: (problem, d, network, hidden widths, N, dt).  The column groups per thread of the
+# forward (TcGeom::ng) are 7 for c2 and d102, 4 for c3, 2 for lqgc7.
+TC_SHAPES = {
+    "c2": ("llgc", 100, "densenet", (30, 30), 10, 0.01),         # C2 / C5: LLGC d = 100, DenseNet [30, 30]
+    "c3": ("dwm", 50, "mlp_tanh", (30, 30), 10, 0.005),          # C3: DoubleWell d = 50 (d_1 = 15, kappa = 5, eta = 3)
+    "lqgc7": ("lqgc", 7, "densenet", (30, 30), 8, 0.02),         # d % 4 != 0
+    "d102": ("llgc", 102, "densenet", (32, 32), 8, 0.01),        # all 512 tensor-memory columns
+}
+
+
+class TcCase:
+    """Inputs of one tensor-core case: K paths from 0, the network, random-sign cotangents with every 7th path exactly
+    zero, the kernels' Philox increments; `oracle()` is the fp64 rollout + gradient (man.grad_mode_a) on them."""
+
+    def __init__(self, abi, shape, K, adaptive=True, wz=False, seed=5, offset=3):
+        kind, d, net, arch, N, dt = TC_SHAPES[shape] if isinstance(shape, str) else shape
+        self.shape, self.kind, self.d, self.net, self.N, self.K = shape, kind, d, net, N, K
+        self.dt, self.adaptive, self.seed, self.offset = np.float32(dt), adaptive, seed, offset
+        self.dims = [d + 1] + list(arch) + [d]
+        self.mp, (self.pid, self.flags, self.pack), self.x0 = hjb_problem(kind, d)
+        cfg = self.cfg()
+        n_theta = abi.lib.pspde_theta_size(ctypes.byref(cfg))
+        assert n_theta > 0, abi.lib.pspde_last_error()
+        rng = np.random.default_rng(seed)
+        self.theta = (0.1 * rng.standard_normal(n_theta)).astype(np.float32)
+        self.wY = (rng.choice([-1.0, 1.0], K) * (0.5 + rng.uniform(0, 1, K)) / K).astype(np.float32)
+        self.wZ = (rng.standard_normal(K) / K).astype(np.float32) if wz else None
+        for w in (self.wY, self.wZ):
+            if w is not None:
+                w[::7] = 0.0
+        self.xi_dump = abi.philox_dump(cfg)                          # (N, K, d)
+        # u_L2 table of the diagnostic, mode 1: u*(x, t_n)_j = tab[2 n, j] + tab[2 n + 1, j] x_j
+        self.table = (0.3 * rng.standard_normal((2 * N, d))).astype(np.float32)
+
+    def cfg(self, K_local=None, k_offset=0, inject=False):
+        strides = (self.d * (self.N + 1), self.N + 1, 1) if inject else (0, 0, 0)
+        return L.make_cfg(self.K if K_local is None else K_local, self.d, self.N, self.dt, self.pid,
+                          L.NET_DENSENET if self.net == "densenet" else L.NET_MLP_TANH, self.dims, L.TIME_FIRST,
+                          adaptive=self.adaptive, k_offset=k_offset, problem_flags=self.flags,
+                          noise_mode=L.NOISE_INJECT if inject else L.NOISE_PHILOX, seed=self.seed, offset=self.offset,
+                          xi_strides=strides)
+
+    def xi_ref(self, lo=0, hi=None):
+        """The Philox increments of paths [lo, hi) in the reference layout (K, d, N + 1), float32."""
+        xi = np.zeros((self.K if hi is None else hi - lo, self.d, self.N + 1), np.float32)
+        xi[:, :, 1:] = self.xi_dump[:, lo:hi].transpose(1, 2, 0)
+        return xi
+
+    def oracle(self, chunk=4096):
+        """fp64: X_N, Y_N, g(X_N), Z_sum and u_L2 per path (u_L2 restates the sum of rollout_tc_fwd_kernel's DIAG build:
+        sum_n dt sum_j (-Z_n,j - u*(X_n+1, t_n)_j)^2), and the gradient of sum_k wY_k Y_N,k + wZ_k Z_sum,k."""
+        key = ("tc", self.shape, self.K, self.adaptive, self.wZ is not None, self.seed, self.offset)
+        if key in _ORACLE:
+            return _ORACLE[key]
+        net = man.Net(self.net, self.dims, self.theta.astype(np.float64))
+        dt = float(self.dt)
+        tab = self.table.astype(np.float64)
+        wZ = np.zeros(self.K) if self.wZ is None else self.wZ.astype(np.float64)
+        parts = []
+        for lo in range(0, self.K, chunk):
+            hi = min(self.K, lo + chunk)
+            g, ro = man.grad_mode_a(self.mp, net, self.xi_ref(lo, hi).astype(np.float64), dt, self.N,
+                                    self.x0.astype(np.float64), self.wY[lo:hi].astype(np.float64), wZ[lo:hi],
+                                    self.adaptive, "first")
+            ul = np.zeros(hi - lo)
+            for n in range(self.N):
+                u = tab[2 * n] + tab[2 * n + 1] * ro["path"][n + 1]
+                ul += dt * ((-ro["Z"][n] - u) ** 2).sum(1)
+            parts.append(dict(grad=g, X=ro["X"], Y=ro["Y"], gX=ro["gX"], Zsum=ro["Zsum"], uL2=ul))
+        out = {k: np.concatenate([p[k] for p in parts]) for k in parts[0] if k != "grad"}
+        out["grad"] = sum(p["grad"] for p in parts)
+        _ORACLE[key] = out
+        return out
+
+    def blocks(self):
+        return grad_blocks(self.net, self.dims)
+
+
+def check_tc_forward(o, m, tol_end=TOL_END):
+    """Per-path outputs of a tensor-core forward against the oracle, and its stats."""
+    assert relerr(o["X"], m["X"]) < tol_end, ("X_N", relerr(o["X"], m["X"]))
+    for k in ("Y", "gX", "Zsum"):
+        assert relerr(o[k], m[k]) < TOL_PATH, (k, relerr(o[k], m[k]))
+    check_stats(o)
+
+
+def check_stats(o):
+    """The stats vector (sum D, sum D^2, sum Z_sum + g, dropped paths; D = Y_N - g(X_N)) against a host recomputation
+    from the per-path outputs it was reduced from."""
+    D = o["Y"].astype(np.float64) - o["gX"]
+    ref = np.array([D.sum(), (D * D).sum(), (o["Zsum"].astype(np.float64) + o["gX"]).sum(), 0.0])
+    scale = np.array([np.abs(D).sum(), (D * D).sum(), np.abs(o["Zsum"].astype(np.float64) + o["gX"]).sum(), 1.0])
+    assert np.all(np.abs(o["stats"] - ref) <= 1e-9 * scale), (o["stats"], ref)
