@@ -186,19 +186,37 @@ def net_input(X, n, dt, time_mode):
     return X
 
 
+def step_net(nets, n, dt, t_index=None, dt_net=None):
+    """(network, time index, grid spacing) that step n evaluates: n on the step grid, or t_index[n] on a network grid of
+    spacing dt_net (importance sampling on another grid: Solver.Z_n, solver.py:360-362, rollout_kernels.cuh's n_net /
+    t_net).  In 'outer' mode (nets a list) the parameter set is that index clamped to [0, len(nets) - 1] (:352)."""
+    n_net, dtn = (n, dt) if t_index is None else (int(t_index[n]), dt_net)
+    if isinstance(nets, list):
+        return nets[min(max(n_net, 0), len(nets) - 1)], n_net, dtn
+    return nets, n_net, dtn
+
+
+def start_states(X0, K, dtype):
+    """X_0 of the K paths: one row for all (tiled) or one row per path (pspde_cfg::x0_per_path)."""
+    X0 = np.asarray(X0, dtype)
+    return np.tile(X0, (K, 1)) if X0.ndim == 1 else X0.copy()
+
+
 # ------------------------------------------------------------------ HJB rollout (solver.py:440-489)
-def rollout(problem, nets, xi, dt, N, X0, adaptive=True, y0=0.0, time_mode="first"):
-    """nets: one Net (inner) or a list of N Nets (outer). xi (K,d,N+1). Returns dict with the X path."""
+def rollout(problem, nets, xi, dt, N, X0, adaptive=True, y0=0.0, time_mode="first", t_index=None, dt_net=None):
+    """nets: one Net (inner) or a list of Nets (outer). xi (K,d,N+1). X0 (d,) or (K, d). t_index / dt_net: see
+    step_net. Returns dict with the X path and Fint = sum_n f(X_{n+1}) dt."""
     K = xi.shape[0]
     dtype = xi.dtype
     s = np.sqrt(dtype.type(dt))
-    X = np.tile(np.asarray(X0, dtype), (K, 1))
+    X = start_states(X0, K, dtype)
     Y = np.full(K, y0, dtype)
     Zsum = np.zeros(K, dtype)
+    Fint = np.zeros(K, dtype)
     path, Zs = [X], []
     for n in range(N):
-        net = nets[n] if isinstance(nets, list) else nets
-        Z, _ = net.forward(net_input(X, n, dt, time_mode))
+        net, n_net, dtn = step_net(nets, n, dt, t_index, dt_net)
+        Z, _ = net.forward(net_input(X, n_net, dtn, time_mode))
         c = -Z if adaptive else np.zeros_like(Z)
         x = xi[:, :, n + 1]
         X = X + (problem.b(X) + c @ problem.B.T) * dt + (x @ problem.B.T) * s
@@ -206,9 +224,10 @@ def rollout(problem, nets, xi, dt, N, X0, adaptive=True, y0=0.0, time_mode="firs
         zz = (Z ** 2).sum(1)
         Y = Y + ((0.5 * zz + fX) + (Z * c).sum(1)) * dt + (Z * x).sum(1) * s
         Zsum = Zsum + (0.5 * zz + fX) * dt
+        Fint = Fint + fX * dt
         path.append(X)
         Zs.append(Z)
-    return dict(X=X, Y=Y, Zsum=Zsum, gX=problem.g(X), path=path, Z=Zs)
+    return dict(X=X, Y=Y, Zsum=Zsum, Fint=Fint, gX=problem.g(X), path=path, Z=Zs)
 
 
 def loss_and_weights(loss_method, Y, gX, Zsum, adaptive=True):
@@ -231,19 +250,21 @@ def loss_and_weights(loss_method, Y, gX, Zsum, adaptive=True):
     raise ValueError(loss_method)
 
 
-def grad_mode_a(problem, nets, xi, dt, N, X0, wY, wZ, adaptive=True, time_mode="first", y0=0.0):
-    """SURVEY.md A.3 generalised: detached forward, one VJP per (k, n)."""
+def grad_mode_a(problem, nets, xi, dt, N, X0, wY, wZ, adaptive=True, time_mode="first", y0=0.0, t_index=None,
+                dt_net=None):
+    """SURVEY.md A.3 generalised: detached forward, one VJP per (k, n).  X0, t_index, dt_net: as in rollout."""
     dtype = xi.dtype
     s = np.sqrt(dtype.type(dt))
-    ro = rollout(problem, nets, xi, dt, N, X0, adaptive, y0, time_mode)
+    ro = rollout(problem, nets, xi, dt, N, X0, adaptive, y0, time_mode, t_index, dt_net)
     outer = isinstance(nets, list)
-    grads = [0.0] * (N if outer else 1)
+    grads = [0.0] * (len(nets) if outer else 1)
     for n in range(N):
-        net = nets[n] if outer else nets
-        Z, tape = net.forward(net_input(ro["path"][n], n, dt, time_mode))
+        net, n_net, dtn = step_net(nets, n, dt, t_index, dt_net)
+        Z, tape = net.forward(net_input(ro["path"][n], n_net, dtn, time_mode))
         zeta = wY[:, None] * (s * xi[:, :, n + 1] + (0.0 if adaptive else 1.0) * Z * dt) + wZ[:, None] * Z * dt
         g = net.vjp(tape, zeta)
-        grads[n if outer else 0] = grads[n if outer else 0] + g
+        i = min(max(n_net, 0), len(nets) - 1) if outer else 0
+        grads[i] = grads[i] + g
     return np.concatenate([np.atleast_1d(g) for g in grads]), ro
 
 

@@ -135,21 +135,21 @@ class Abi:
         return self.host(X0), self.host(t0)
 
     # -- tensor-core rollout and gradient kernels (device only: tcgen05 has no host emulation)
-    def fwd_ckpt(self, cfg, theta, pack, x0, xi=None, table=None, ckpt_bytes=0):
+    def fwd_ckpt(self, cfg, theta, pack, x0, xi=None, table=None, ckpt_bytes=0, y0=None):
         """pspde_rollout_fwd_ckpt: the forward, with the u_L2 diagnostic (mode 1, linear table) if `table` is given and
-        keeping the operand rows of its first tiles in a buffer of ckpt_bytes if that is > 0.  Returns (outputs,
-        device checkpoint buffer or None, launches it took)."""
+        keeping the operand rows of its first tiles in a buffer of ckpt_bytes if that is > 0; y0 (a float) is Y's
+        start value.  Returns (outputs, device checkpoint buffer or None, launches it took)."""
         K, d = cfg.K_local, cfg.d
         ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
         o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4, uL2=K))
-        ins = [self.dev(a) for a in (theta, pack, x0, xi, table)]
+        ins = [self.dev(a) for a in (theta, pack, x0, xi, table, None if y0 is None else [y0])]
         diag = None
         if table is not None:
             diag = L.pspde_udiag(mode=1, nx1=0, d1=0, xb=0.0, dx=0.0, table=ins[4].data_ptr(), uL2=o["uL2"].data_ptr(),
                                  quirk_path=-1)
         ck = self.zeros(ckpt_bytes // 4) if ckpt_bytes else None
         n0 = self.lib.pspde_launch_count()
-        rc = self.lib.pspde_rollout_fwd_ckpt(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], None, self.xi_ptr(ins[3]),
+        rc = self.lib.pspde_rollout_fwd_ckpt(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], self.p(ins[5]), self.xi_ptr(ins[3]),
                                              self.p(o["X"]), self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]),
                                              self.p(o["stats"]), None if diag is None else ctypes.byref(diag), self.p(ck),
                                              ckpt_bytes, self.p(ws), self.nbytes(ws), None)
@@ -171,6 +171,20 @@ class Abi:
                                                  None)
         L.check(self.lib, rc)
         return self.host(grad), self.lib.pspde_launch_count() - n0
+
+    def importance_sampling(self, cfg, theta, pack, x0, t_index=None, dt_net=0.0):
+        """pspde_importance_sampling (network time index t_index[n] on a grid of spacing dt_net, if given): (outputs
+        X, Y, gX, Fint, launches it took)."""
+        K, d = cfg.K_local, cfg.d
+        ws = self.ws(self.lib.pspde_workspace_bytes_fwd(ctypes.byref(cfg)))
+        o = self._out(dict(X=(K, d), Y=K, gX=K, Fint=K))
+        ins = [self.dev(a) for a in (theta, pack, x0)] + [self.dev(t_index, np.int32)]
+        n0 = self.lib.pspde_launch_count()
+        rc = self.lib.pspde_importance_sampling(ctypes.byref(cfg), *[self.p(a) for a in ins[:3]], None, self.p(ins[3]),
+                                                ctypes.c_float(dt_net), self.p(o["X"]), self.p(o["Y"]), self.p(o["gX"]),
+                                                self.p(o["Fint"]), self.p(ws), self.nbytes(ws), None)
+        L.check(self.lib, rc)
+        return self._host_all(o), self.lib.pspde_launch_count() - n0
 
     def grad_from_fwd_ckpt(self, cfg, theta, pack, x0, ck, wY, xi=None):
         """pspde_grad_from_fwd_ckpt on the rows a fwd_ckpt call kept: (gradient, launches it took)."""
@@ -439,12 +453,13 @@ class TcCase:
     """Inputs of one tensor-core case: K paths from 0, the network, random-sign cotangents with every 7th path exactly
     zero, the kernels' Philox increments; `oracle()` is the fp64 rollout + gradient (man.grad_mode_a) on them."""
 
-    def __init__(self, abi, shape, K, adaptive=True, wz=False, seed=5, offset=3):
+    def __init__(self, abi, shape, K, adaptive=True, wz=False, seed=5, offset=3, x0_per_path=False, y0=None):
         kind, d, net, arch, N, dt = TC_SHAPES[shape] if isinstance(shape, str) else shape
         self.shape, self.kind, self.d, self.net, self.N, self.K = shape, kind, d, net, N, K
         self.dt, self.adaptive, self.seed, self.offset = np.float32(dt), adaptive, seed, offset
         self.dims = [d + 1] + list(arch) + [d]
         self.mp, (self.pid, self.flags, self.pack), self.x0 = hjb_problem(kind, d)
+        self.y0 = y0
         cfg = self.cfg()
         n_theta = abi.lib.pspde_theta_size(ctypes.byref(cfg))
         assert n_theta > 0, abi.lib.pspde_last_error()
@@ -458,6 +473,8 @@ class TcCase:
         self.xi_dump = abi.philox_dump(cfg)                          # (N, K, d)
         # u_L2 table of the diagnostic, mode 1: u*(x, t_n)_j = tab[2 n, j] + tab[2 n + 1, j] x_j
         self.table = (0.3 * rng.standard_normal((2 * N, d))).astype(np.float32)
+        if x0_per_path:                                              # one start point per path around the problem's X_0
+            self.x0 = (self.x0 + 0.5 * rng.standard_normal((K, d))).astype(np.float32)
 
     def cfg(self, K_local=None, k_offset=0, inject=False):
         strides = (self.d * (self.N + 1), self.N + 1, 1) if inject else (0, 0, 0)
@@ -465,7 +482,7 @@ class TcCase:
                           L.NET_DENSENET if self.net == "densenet" else L.NET_MLP_TANH, self.dims, L.TIME_FIRST,
                           adaptive=self.adaptive, k_offset=k_offset, problem_flags=self.flags,
                           noise_mode=L.NOISE_INJECT if inject else L.NOISE_PHILOX, seed=self.seed, offset=self.offset,
-                          xi_strides=strides)
+                          xi_strides=strides, x0_per_path=self.x0.ndim == 2)
 
     def xi_ref(self, lo=0, hi=None):
         """The Philox increments of paths [lo, hi) in the reference layout (K, d, N + 1), float32."""
@@ -476,19 +493,20 @@ class TcCase:
     def oracle(self, chunk=4096):
         """fp64: X_N, Y_N, g(X_N), Z_sum and u_L2 per path (u_L2 restates the sum of rollout_tc_fwd_kernel's DIAG build:
         sum_n dt sum_j (-Z_n,j - u*(X_n+1, t_n)_j)^2), and the gradient of sum_k wY_k Y_N,k + wZ_k Z_sum,k."""
-        key = ("tc", self.shape, self.K, self.adaptive, self.wZ is not None, self.seed, self.offset)
+        key = ("tc", self.shape, self.K, self.adaptive, self.wZ is not None, self.seed, self.offset, self.x0.ndim, self.y0)
         if key in _ORACLE:
             return _ORACLE[key]
         net = man.Net(self.net, self.dims, self.theta.astype(np.float64))
         dt = float(self.dt)
         tab = self.table.astype(np.float64)
         wZ = np.zeros(self.K) if self.wZ is None else self.wZ.astype(np.float64)
+        x0 = self.x0.astype(np.float64)
         parts = []
         for lo in range(0, self.K, chunk):
             hi = min(self.K, lo + chunk)
             g, ro = man.grad_mode_a(self.mp, net, self.xi_ref(lo, hi).astype(np.float64), dt, self.N,
-                                    self.x0.astype(np.float64), self.wY[lo:hi].astype(np.float64), wZ[lo:hi],
-                                    self.adaptive, "first")
+                                    x0[lo:hi] if x0.ndim == 2 else x0, self.wY[lo:hi].astype(np.float64), wZ[lo:hi],
+                                    self.adaptive, "first", float(np.float32(self.y0 or 0.0)))
             ul = np.zeros(hi - lo)
             for n in range(self.N):
                 u = tab[2 * n] + tab[2 * n + 1] * ro["path"][n + 1]

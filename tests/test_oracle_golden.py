@@ -181,6 +181,57 @@ def test_importance_sampling_port(tag):
     assert abs(v - g["var"]) < 1e-4 * abs(g["var"])
 
 
+@pytest.mark.parametrize("tag", ["is_llgc_d10_dense", "is_dwm_d4_mlp"])
+def test_manual_rollout_on_network_grid(tag):
+    """man.rollout with the network evaluated at t_index[n] dt_net (t_index[n] = ceil(n dt / dt_net), the fp32 division of
+    Solver.Z_n) reproduces the reference's importance-sampling mean and variance, w = exp(Y_N - 2 Fint - g(X_N))."""
+    g = load_golden(tag)
+    d, dt, dt_net = g["d"], g["is_dt"], g["solver_dt"]
+    g["time_approx"] = "inner"
+    dims = net_dims(g)
+    p32 = orc.make_problem(g["kind"], d, **g["pkw"])
+    if g["kind"] == "dwm":
+        prob = man.Problem("dwm", d, eta_=p32.eta_.numpy(), kappa_=p32.kappa_.numpy())
+    else:
+        prob = man.Problem(g["kind"], d, A=p32.A.numpy(), B=p32.B.numpy())
+    N, K = g["xis"].shape[:2]
+    xi = np.zeros((K, d, N + 1))
+    xi[:, :, 1:] = g["xis"].transpose(1, 2, 0)
+    t_index = [int(np.ceil(np.float32(n * dt) / np.float32(dt_net))) for n in range(N)]
+    assert t_index != list(range(N))                  # a coarser (llgc) or finer (dwm) network grid: the remap matters
+    ro = man.rollout(prob, man.Net(g["net"], dims, g["theta"]), xi, dt, N, p32.X_0.numpy(), True, 0.0, "first",
+                     t_index, dt_net)
+    w = np.exp(ro["Y"] - 2 * ro["Fint"] - ro["gX"])
+    assert abs(w.mean() - g["mean"]) < 1e-5 * abs(g["mean"])
+    assert abs(w.var(ddof=1) - g["var"]) < 1e-4 * abs(g["var"])
+
+
+@pytest.mark.parametrize("tag", ["hjb_lqgc_d10_dense_lv", "hjb_lqgc_d10_outer_lv"])
+def test_manual_extensions_reduce_to_the_pinned_oracle(tag):
+    """The per-path X_0 and network-time arguments of man.rollout / man.grad_mode_a: a tiled X_0 and t_index = arange(N)
+    with dt_net = dt give the one-row, step-grid result bit for bit."""
+    g = load_golden(tag)
+    d, N, dt = g["d"], g["N"], g["delta_t"]
+    outer = g["time_approx"] == "outer"
+    per = g["theta"].size // (N if outer else 1)
+    nets = [man.Net(g["net"], net_dims(g), g["theta"][i * per:(i + 1) * per]) for i in range(N if outer else 1)]
+    nets = nets if outer else nets[0]
+    prob, tm = man.Problem(g["kind"], d, A=g["A"], B=g["B"]), "none" if outer else "first"
+    xi = g["xi"].astype(np.float64)
+    K = xi.shape[0]
+    X0 = 0.1 * np.arange(d)
+    wY, wZ = np.linspace(-1, 1, K) / K, np.linspace(0, 1, K) / K
+    ref = man.grad_mode_a(prob, nets, xi, dt, N, X0, wY, wZ, g["adaptive"], tm, 0.5)
+    for kw in (dict(X0=np.tile(X0, (K, 1))), dict(t_index=np.arange(N), dt_net=dt)):
+        args = dict(X0=X0, t_index=None, dt_net=None)
+        args.update(kw)
+        got = man.grad_mode_a(prob, nets, xi, dt, N, args["X0"], wY, wZ, g["adaptive"], tm, 0.5, args["t_index"],
+                              args["dt_net"])
+        assert np.array_equal(got[0], ref[0])
+        for k in ("X", "Y", "Zsum", "Fint", "gX"):
+            assert np.array_equal(got[1][k], ref[1][k]), k
+
+
 LOOPS = {
     "loop_G1": dict(kind="lqgc", d=10, pkw={}, net="densenet", ta="outer", K=200, dt=0.05, L=3, lr=1e-3,
                     loss="log-variance", detach=True),
