@@ -82,17 +82,32 @@ class Abi:
         L.check(self.lib, rc)
         return self._host_all(o)
 
-    def attached(self, cfg, theta, pack, x0, w, wY=None, wZ=None, wG=None):
+    def addr(self, a):
+        return a.ctypes.data if self.device is None else a.data_ptr()
+
+    def attached(self, cfg, theta, pack, x0, w, wY=None, wZ=None, wG=None, y0=None, xi=None, table=None):
+        """pspde_rollout_attached: relative entropy in one launch (w, no per-path cotangents) or per-path cotangents;
+        y0 (a float) is Y's start value, xi the injected increments in the reference layout (K, d, N + 1).  With a
+        `table` it calls pspde_rollout_attached_diag with the u_L2 diagnostic (mode 1, linear table).  Returns
+        (outputs, launches it took)."""
         K, d = cfg.K_local, cfg.d
         ws = self.ws(self.lib.pspde_workspace_bytes(ctypes.byref(cfg)))
-        o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4, grad=self.lib.pspde_theta_size(ctypes.byref(cfg))))
-        keep = [self.dev(a) for a in (theta, pack, x0, wY, wZ, wG)]
-        rc = self.lib.pspde_rollout_attached(ctypes.byref(cfg), *[self.p(a) for a in keep[:3]], None, None,
-                                             ctypes.c_float(w), *[self.p(a) for a in keep[3:]], self.p(o["X"]),
-                                             self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]), self.p(o["stats"]),
-                                             self.p(o["grad"]), self.p(ws), self.nbytes(ws), None)
+        o = self._out(dict(X=(K, d), Y=K, gX=K, Zsum=K, stats=4, grad=self.lib.pspde_theta_size(ctypes.byref(cfg)),
+                           uL2=K))
+        keep = [self.dev(a) for a in (theta, pack, x0, None if y0 is None else [y0], xi, wY, wZ, wG, table)]
+        args = [ctypes.byref(cfg), *[self.p(a) for a in keep[:4]], self.xi_ptr(keep[4]), ctypes.c_float(w),
+                *[self.p(a) for a in keep[5:8]], self.p(o["X"]), self.p(o["Y"]), self.p(o["gX"]), self.p(o["Zsum"]),
+                self.p(o["stats"])]
+        tail = [self.p(o["grad"]), self.p(ws), self.nbytes(ws), None]
+        n0 = self.lib.pspde_launch_count()
+        if table is None:
+            rc = self.lib.pspde_rollout_attached(*args, *tail)
+        else:
+            diag = L.pspde_udiag(mode=1, nx1=0, d1=0, xb=0.0, dx=0.0, table=self.addr(keep[8]), uL2=self.addr(o["uL2"]),
+                                 quirk_path=-1)
+            rc = self.lib.pspde_rollout_attached_diag(*args, ctypes.byref(diag), *tail)
         L.check(self.lib, rc)
-        return self._host_all(o)
+        return self._host_all(o), self.lib.pspde_launch_count() - n0
 
     # -- diffusion / elliptic
     def diff_fwd(self, cfg, T, theta, pack, X0, t0, xis, ell=None):
@@ -158,7 +173,9 @@ class Abi:
 
     def xi_ptr(self, xi):
         """Injected increments in the reference layout (K, d, N + 1): slice n + 1 drives step n."""
-        return None if xi is None else ctypes.c_void_p(xi.data_ptr() + 4 * xi.stride(2))
+        if xi is None:
+            return None
+        return ctypes.c_void_p(xi.ctypes.data + xi.strides[2] if self.device is None else xi.data_ptr() + 4 * xi.stride(2))
 
     def bwd_detached(self, cfg, theta, pack, x0, wY, wZ=None, xi=None):
         """pspde_rollout_bwd_detached: (gradient, launches it took)."""
@@ -280,7 +297,7 @@ def attached_case(abi, kind, d, net, K, N, dt, loss, off_diag=0.0, outer=False, 
     xi[:, :, 1:] = abi.philox_dump(cfg).transpose(1, 2, 0)
     mode = "none" if outer else "first"
     if loss == "relative_entropy":
-        o = abi.attached(cfg, theta, pack, x0, 1.0 / K)
+        o, _ = abi.attached(cfg, theta, pack, x0, 1.0 / K)
         gm, ro = man.grad_mode_b(mp, nets[0], xi, dt, N, x0.astype(np.float64), mode)
     else:
         f = abi.fwd(cfg, theta, pack, x0)
@@ -290,7 +307,7 @@ def attached_case(abi, kind, d, net, K, N, dt, loss, off_diag=0.0, outer=False, 
         if inert:
             for w in (wY, wZ, wG):
                 w[::7] = 0.0
-        o = abi.attached(cfg, theta, pack, x0, 0.0, wY, wZ, wG)
+        o, _ = abi.attached(cfg, theta, pack, x0, 0.0, wY, wZ, wG)
         gm, ro = man.grad_attached(mp, nets if outer else nets[0], xi, dt, N, x0.astype(np.float64),
                                    wY.astype(np.float64), wZ.astype(np.float64), wG.astype(np.float64), mode)
         for k in ("X", "Y", "Zsum", "gX"):           # the forward launch that produced the cotangents
@@ -491,14 +508,12 @@ class TcCase:
         return xi
 
     def oracle(self, chunk=4096):
-        """fp64: X_N, Y_N, g(X_N), Z_sum and u_L2 per path (u_L2 restates the sum of rollout_tc_fwd_kernel's DIAG build:
-        sum_n dt sum_j (-Z_n,j - u*(X_n+1, t_n)_j)^2), and the gradient of sum_k wY_k Y_N,k + wZ_k Z_sum,k."""
+        """fp64: X_N, Y_N, g(X_N), Z_sum and u_L2 per path (u_l2), and the gradient of sum_k wY_k Y_N,k + wZ_k Z_sum,k."""
         key = ("tc", self.shape, self.K, self.adaptive, self.wZ is not None, self.seed, self.offset, self.x0.ndim, self.y0)
         if key in _ORACLE:
             return _ORACLE[key]
         net = man.Net(self.net, self.dims, self.theta.astype(np.float64))
         dt = float(self.dt)
-        tab = self.table.astype(np.float64)
         wZ = np.zeros(self.K) if self.wZ is None else self.wZ.astype(np.float64)
         x0 = self.x0.astype(np.float64)
         parts = []
@@ -507,11 +522,7 @@ class TcCase:
             g, ro = man.grad_mode_a(self.mp, net, self.xi_ref(lo, hi).astype(np.float64), dt, self.N,
                                     x0[lo:hi] if x0.ndim == 2 else x0, self.wY[lo:hi].astype(np.float64), wZ[lo:hi],
                                     self.adaptive, "first", float(np.float32(self.y0 or 0.0)))
-            ul = np.zeros(hi - lo)
-            for n in range(self.N):
-                u = tab[2 * n] + tab[2 * n + 1] * ro["path"][n + 1]
-                ul += dt * ((-ro["Z"][n] - u) ** 2).sum(1)
-            parts.append(dict(grad=g, X=ro["X"], Y=ro["Y"], gX=ro["gX"], Zsum=ro["Zsum"], uL2=ul))
+            parts.append(dict(grad=g, X=ro["X"], Y=ro["Y"], gX=ro["gX"], Zsum=ro["Zsum"], uL2=u_l2(self.table, ro, dt)))
         out = {k: np.concatenate([p[k] for p in parts]) for k in parts[0] if k != "grad"}
         out["grad"] = sum(p["grad"] for p in parts)
         _ORACLE[key] = out
@@ -519,6 +530,17 @@ class TcCase:
 
     def blocks(self):
         return grad_blocks(self.net, self.dims)
+
+
+def u_l2(table, ro, dt):
+    """The u_L2 diagnostic of mode 1 (u*(x, t_n)_j = table[2 n, j] + table[2 n + 1, j] x_j) on an oracle rollout ro, as
+    the forward sweeps sum it (solver.py:491-494): sum_n dt sum_j (-Z_n,j - u*(X_n+1, t_n)_j)^2 per path."""
+    tab = table.astype(np.float64)
+    ul = 0.0
+    for n in range(len(ro["Z"])):
+        u = tab[2 * n] + tab[2 * n + 1] * ro["path"][n + 1]
+        ul = ul + dt * ((-ro["Z"][n] - u) ** 2).sum(1)
+    return ul
 
 
 def check_tc_forward(o, m, tol_end=TOL_END):
