@@ -266,6 +266,7 @@ int pspde_diffusion_fwd(const pspde_cfg* cfg, float T_end, const float* theta, c
  * (they do not depend on theta) and every step runs the reverse of the (value, tangent) pair.  Per-path
  * cotangents (length K_local, nullable = 0): c0 = dL/dV(X_0, t_0), cD = dL/d(each active directional derivative),
  * cE = dL/dV(X_end, t_end).  For loss = alpha_0 mean(r^2): w = 2 alpha_0 r / K, c0 = cD = -w, cE = w.
+ * A path with all-zero cotangents is inert, even if it diverged (GeneralSolver drops a path with a non-finite r this way).
  * grad_theta (pspde_theta_size floats) is overwritten. */
 int pspde_diffusion_bwd(const pspde_cfg* cfg, float T_end, const float* theta, const float* prob, const float* X0,
                         const float* t0, const float* xi, const float* c0, const float* cE, const float* cD,
@@ -299,7 +300,8 @@ int pspde_diffusion_bwd(const pspde_cfg* cfg, float T_end, const float* theta, c
  * a path entered un-stopped of (V(X_n) - v_true(X_n))^2 dt (all nullable).  stats as in pspde_diffusion_fwd.
  * With N = 0 it evaluates V at X0 (the Dirichlet boundary term of :669-670 is this call on the boundary samples).
  * pspde_elliptic_bwd -- cotangents as in pspde_diffusion_bwd; the value row of step n additionally receives
- * cD act (-dh/dy(X_n, V(X_n)) dt).  INJECT strides as in pspde_diffusion_fwd. */
+ * cD act (-dh/dy(X_n, V(X_n)) dt); a path with all-zero cotangents is inert, even if it diverged.  INJECT strides as in
+ * pspde_diffusion_fwd. */
 enum { PSPDE_DOMAIN_SPHERE = 1, PSPDE_DOMAIN_BOX = 2, PSPDE_DOMAIN_ANNULUS = 3 };
 enum { PSPDE_H_ZERO = 0, PSPDE_H_EXP_LINEAR = 1, PSPDE_H_EXP_NONLINEAR = 2, PSPDE_H_EXP_NONLINEAR_SIN = 3,
        PSPDE_H_HELMHOLTZ = 4, PSPDE_H_COMMITTOR = 6 };

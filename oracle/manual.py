@@ -328,13 +328,27 @@ def grad_attached(problem, nets, xi, dt, N, X0, wY, wZ, wG, time_mode="first", y
 
 
 # ------------------------------------------------------------------ diffusion loss (solver.py:1062-1163, h == 0)
+def _path_grad(grad, net, tape0, tapeE, steps, dt, cot):
+    """grad + the theta-gradient of sum_k c0 V(X_0) + cE V(X_end) + sum_n cD act (directional derivative - h dt): the
+    value row of an active step gets cD act (-h_y dt), the tangent row cD act."""
+    c0, cE, cD = cot
+    grad = grad + net.vjp(tapeE, cE[:, None]) + net.vjp(tape0, c0[:, None])
+    for tape, act, hy in steps:
+        grad = grad + net.vjp_tangent(tape, (-cD * act * hy * dt)[:, None], (cD * act)[:, None])
+    return grad
+
+
 ALLEN_CAHN = dict(h=lambda y: y - y ** 3, h_y=lambda y: 1 - 3 * y ** 2, f=lambda x: 1 / (2 + 2 / 5 * (x ** 2).sum(1)))
 
 
-def diffusion(problem, net, X0, t0, xis, dt, N, K_boundary, alpha=(1.0, 1.0, 1.0), T=1.0, pde=None):
+def diffusion(problem, net, X0, t0, xis, dt, N, K_boundary, alpha=(1.0, 1.0, 1.0), T=1.0, pde=None, cot=None):
     """Value and theta-gradient of the diffusion loss, unbounded domain, non-adaptive; net input is [X, t].
+    The process is X += (b(X) dt + B xi sqrt(dt)) act with the problem's drift and sigma: Problem('heat', d) (b = 0,
+    sigma = sqrt(2) I) or Problem('llgc', d, A=diag(a), B=diag(b)) (the kernels' PSPDE_PROBLEM_OU pack a_diag | b_diag).
     pde = None: heat equation (h == 0, terminal |x|^2); pde = ALLEN_CAHN: h(y) = y - y^3, the value row of every
-    active step then carries the cotangent w act h_y dt (as in `elliptic` below)."""
+    active step then carries the cotangent w act h_y dt (as in `elliptic` below).
+    cot = (c0, cE, cD): per-path cotangents on V(X_0, t_0), V(X_end, t_end) and every active directional derivative
+    (pspde_diffusion_bwd) in place of the loss's (-w, w, -w); the terminal-condition term is added either way."""
     dtype = X0.dtype
     K, d = X0.shape
     dt = dtype.type(np.float32(dt))
@@ -376,19 +390,19 @@ def diffusion(problem, net, X0, t0, xis, dt, N, K_boundary, alpha=(1.0, 1.0, 1.0
     r = vE[:, 0] - Y
     loss = loss + alpha[0] * (r ** 2).mean()
     w = alpha[0] * 2 * r / K
-    grad = grad + net.vjp(tapeE, w[:, None]) - net.vjp(tape0, w[:, None])
-    for tape, act, hy in steps:
-        grad = grad + net.vjp_tangent(tape, (w * act * hy * dt)[:, None], (-w * act)[:, None])
+    grad = _path_grad(grad, net, tape0, tapeE, steps, dt, (-w, w, -w) if cot is None else cot)
     return dict(loss=loss, grad=grad, K_count=K_count, X=X, t=t, Y=Y)
 
 
 # ------------------------------------------------------------------ elliptic diffusion loss (solver.py:628-790)
 class EllipticProblem:
-    """numpy functors of the elliptic problems (problems.py:962-1064, :1614-1654): b = 0, sigma = sqrt(2) I,
-    h(x, y) with its y-derivative, Dirichlet data g, exact solution v_true."""
+    """numpy functors of the elliptic problems (problems.py:962-1064, :1614-1654): b = 0, sigma = sqrt(2) I (committor:
+    I), h(x, y) with its y-derivative, Dirichlet data g, exact solution v_true.  a, b (length d): a diagonal drift
+    b(x) = a x and sigma = diag(b) instead, as the kernels take them from the problem pack (a_diag | b_diag)."""
 
-    def __init__(self, kind, d, alpha=1.0, dtype=np.float64):
+    def __init__(self, kind, d, alpha=1.0, dtype=np.float64, a=None, b=None):
         self.kind, self.d, self.alpha, self.dtype = kind, d, float(alpha), dtype
+        self.a = np.zeros(d, dtype) if a is None else np.asarray(a, dtype)
         self.B = np.sqrt(dtype(2.0)) * np.eye(d, dtype=dtype)
         if kind == "helmholtz":
             self.boundary, self.one_boundary, self.X_l, self.X_r = "square", False, -1.0, 1.0
@@ -398,6 +412,8 @@ class EllipticProblem:
             self.B = np.eye(d, dtype=dtype)
         else:
             self.boundary, self.boundary_distance = "sphere", 1.0
+        if b is not None:
+            self.B = np.diag(np.asarray(b, dtype))
 
     def _ss(self, x):
         return np.sin(self.a_1 * np.pi * x[:, 0]) * np.sin(self.a_2 * np.pi * x[:, 1])
@@ -449,11 +465,12 @@ class EllipticProblem:
         return ((X_prop >= self.X_l) & (X_prop <= self.X_r)).all(1)
 
 
-def elliptic(problem, net, Xb, X0, xis, dt, N, alpha=(1.0, 1.0), gb=None):
+def elliptic(problem, net, Xb, X0, xis, dt, N, alpha=(1.0, 1.0), gb=None, cot=None):
     """Value and theta-gradient of the elliptic diffusion loss (non-adaptive, Dirichlet term); net input is X.
+    The proposal of step n is X_n + (a X_n dt + v_n), v_n = B xi_n sqrt(dt), as the kernels form it.
         Y = V(X_0) + sum_n act_n (-h(X_n, V(X_n)) dt + grad V(X_n) . B xi_n sqrt(dt)),  r = V(X_end) - Y
         dL = sum_k w_k [dV(X_end) - dV(X_0) + sum_n act_n (h_y dt dV(X_n) - d(grad V(X_n) . v_n))],  w = 2 alpha_0 r / K
-    i.e. per step the (value, tangent) pair gets the cotangents (w act h_y dt, -w act)."""
+    i.e. per step the (value, tangent) pair gets the cotangents (w act h_y dt, -w act).  cot: as in `diffusion`."""
     dtype = X0.dtype
     K, d = X0.shape
     dt = dtype.type(np.float32(dt))
@@ -476,7 +493,7 @@ def elliptic(problem, net, Xb, X0, xis, dt, N, alpha=(1.0, 1.0), gb=None):
         y, dy, tape = net.forward_tangent(X, v)
         sel = ~stopped
         V_L2 += (y[:, 0] - problem.v_true(X)) ** 2 * dt * sel
-        X_prop = X + v * sel[:, None]
+        X_prop = X + ((problem.a * X) * dt + v) * sel[:, None]
         act = problem.inside(X, X_prop) & ~stopped
         Y = Y + (-problem.h(X, y[:, 0]) * dt + dy[:, 0]) * act
         steps.append((tape, act.copy(), problem.h_y(X, y[:, 0])))
@@ -487,7 +504,5 @@ def elliptic(problem, net, Xb, X0, xis, dt, N, alpha=(1.0, 1.0), gb=None):
     r = vE[:, 0] - Y
     loss = loss_b + alpha[0] * (r ** 2).mean()
     w = alpha[0] * 2 * r / K
-    grad = grad + net.vjp(tapeE, w[:, None]) - net.vjp(tape0, w[:, None])
-    for tape, act, hy in steps:
-        grad = grad + net.vjp_tangent(tape, (w * act * hy * dt)[:, None], (-w * act)[:, None])
+    grad = _path_grad(grad, net, tape0, tapeE, steps, dt, (-w, w, -w) if cot is None else cot)
     return dict(loss=loss, loss_boundary=loss_b, grad=grad, K_count=K_count, X=X, Y=Y, V_L2=V_L2, r=r)

@@ -16,6 +16,8 @@
 // the gradient is a second launch that regenerates the trajectories (Philox | injected xi) and, per step, runs
 // the reverse of the (value, tangent) pair (oracle/manual.py::Net.vjp_tangent) with the per-path cotangents
 //   c0 on V(X_0, t_0),  cD on every active directional derivative,  cE on V(X_end, t_end).
+// A path whose three cotangents are all zero contributes nothing; the backward keeps it at the origin and stopped, so
+// that a path the caller dropped for a non-finite residual (a diverged X_0) cannot put inf * 0 = NaN into the gradient.
 // The network is too large for shared memory at the C4 size (371 KB of weights): the weights are re-laid once per
 // call into a padded k4-blocked buffer in global memory (L2 resident) and streamed through the read-only path;
 // the weight gradient of one tile-step is accumulated in registers (8x8 blocks over the 2P rows) and added to
@@ -343,13 +345,22 @@ __global__ void __launch_bounds__(T, 1) diffusion_kernel(const DiffusionParams p
   float* gp = BWD ? prm.grad_partial + (size_t)blockIdx.x * dw_partial_floats(g) : nullptr;
   __syncthreads();
 
+  // backward: a path with c0 = cE = cD = 0 (the solvers zero the cotangents of a path whose residual is not finite) is
+  // inert: it starts at the origin and is stopped from step 0, so every activation, h_y and epilogue value it produces
+  // is finite and its zero cotangents add exact zeros to the weight gradient (from a diverged X_0, inf * 0 = NaN would)
+  auto inert = [&](int k) {
+    return BWD && (!prm.c0 || __ldg(prm.c0 + k) == 0.f) && (!prm.cE || __ldg(prm.cE + k) == 0.f) &&
+           (!prm.cD || __ldg(prm.cD + k) == 0.f);
+  };
+
   for (int tile = blockIdx.x; tile < prm.n_tiles; tile += gridDim.x) {
-    // ---- tile init: value rows [X_0 | t_0 | 1 | 0], tangent rows 0 (solver.py:1045-1046, :1078-1081)
+    // ---- tile init: value rows [X_0 | t_0 | 1 | 0] ([0 | t_0 | 1 | 0] for an inert path), tangent rows 0
+    // (solver.py:1045-1046, :1078-1081)
     for (int q = tid; q < P * ngrp0 * 4; q += T) {
       const int p = q / (ngrp0 * 4), j = q - p * ngrp0 * 4, k = tile * P + p;
       float x = 0.f;
       if (k < prm.K_local) {
-        if (j < d) x = __ldg(prm.X0 + (size_t)k * d + j);
+        if (j < d) x = inert(k) ? 0.f : __ldg(prm.X0 + (size_t)k * d + j);
         else if (j == g.seg_one[0]) x = 1.0f;
       }
       sAct[p * lda + j] = x;
@@ -360,7 +371,7 @@ __global__ void __launch_bounds__(T, 1) diffusion_kernel(const DiffusionParams p
       const bool in = k < prm.K_local;
       sY[p] = 0.f; sA[p] = 0.f; sNA[p] = 0.f; sVL[p] = 0.f;
       sT[p] = (in && prm.t0) ? __ldg(prm.t0 + k) : 0.f;
-      sS[p] = in ? 0.f : 1.f;
+      sS[p] = (in && !inert(k)) ? 0.f : 1.f;
       sC0[p] = (BWD && in && prm.c0) ? __ldg(prm.c0 + k) : 0.f;
       sCE[p] = (BWD && in && prm.cE) ? __ldg(prm.cE + k) : 0.f;
       sCD[p] = (BWD && in && prm.cD) ? __ldg(prm.cD + k) : 0.f;

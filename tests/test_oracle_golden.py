@@ -332,3 +332,40 @@ def test_elliptic_training_loop_pins(tag, kind, d, N):
     ll, kc = orc.elliptic_train_loop(orc.make_problem(kind, d), params, 200, 50, N, 1e-3, 3, 1e-3, seed=42)
     np.testing.assert_allclose(ll, g["loss_log"], rtol=2e-6)
     assert kc == [int(v) for v in g["K_log"]]
+
+
+@pytest.mark.parametrize("tag", ["diff_heat_d10_small", "diff_allencahn_d20"] + ELL_TAGS)
+def test_drift_sigma_and_cotangent_forms_reproduce_the_oracle(tag):
+    """The forms the kernel tests use reproduce the oracle's results on the reference's goldens bit for bit: `diffusion`
+    on Problem('llgc', A = 0, B = sqrt(2) I) and `elliptic` with a = 0 and b = sqrt(2) (committor: 1) equal the
+    default problems, and explicit per-path cotangents (c0, cE, cD) = (-w, w, -w) equal the loss's own."""
+    g = load_golden(tag)
+    d = int(g["d"])
+    arch = [int(a) for a in g["arch"]]
+    if tag.startswith("diff"):
+        dims = [d + 1] + arch + [1]
+        net = man.Net("densenet", dims, g["theta"])
+        X0, t0, xis = (g[k].astype(np.float64) for k in ("X0", "t0", "xis"))
+        alpha = tuple(float(a) for a in g["alpha"]) if "alpha" in g else (1.0, 1.0, 1.0)
+        kw = dict(alpha=alpha, T=float(g["T"]) if "T" in g else 1.0, pde=man.ALLEN_CAHN if "allencahn" in tag else None)
+        run = lambda prob, **k: man.diffusion(prob, net, X0, t0, xis, g["delta_t"], int(g["N"]), int(g["K_boundary"]),
+                                              **kw, **k)
+        m = run(man.Problem("heat", d))
+        same = run(man.Problem("llgc", d, A=np.zeros((d, d)), B=np.sqrt(2.0) * np.eye(d)))
+        r = net.forward(np.concatenate([m["X"], m["t"][:, None]], 1))[0][:, 0] - m["Y"]
+    else:
+        kind = str(g["kind"])
+        net = man.Net("densenet", [d] + arch + [1], g["theta"])
+        alpha = tuple(float(a) for a in g["alpha"])
+        gb = orc.make_problem(kind, d).g(pt.tensor(g["Xb"])).numpy().astype(np.float64)
+        run = lambda prob, **k: man.elliptic(prob, net, g["Xb"].astype(np.float64), g["X0"].astype(np.float64),
+                                             g["xis"].astype(np.float64), g["delta_t"], int(g["N"]), alpha, gb=gb, **k)
+        m = run(man.EllipticProblem(kind, d))
+        b = np.ones(d) if kind == "committor" else np.full(d, np.sqrt(2.0))
+        same = run(man.EllipticProblem(kind, d, a=np.zeros(d), b=b))
+        r = m["r"]
+    for k in m:
+        assert np.array_equal(m[k], same[k]), k
+    w = alpha[0] * 2 * r / r.size
+    assert np.array_equal(run(man.Problem("heat", d) if tag.startswith("diff") else man.EllipticProblem(str(g["kind"]), d),
+                              cot=(-w, w, -w))["grad"], m["grad"])
