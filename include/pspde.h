@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define PSPDE_ABI_VERSION 2
+#define PSPDE_ABI_VERSION 3
 #define PSPDE_MAX_LAYERS 4          /* linear layers per network (<= 3 hidden) */
 
 /* problem functors (problems.py): drift b(x), diffusion sigma = B, running cost f, terminal cost g.
@@ -203,6 +203,58 @@ int pspde_lv_cotangents(int K_local, double K_global, int moment, const float* Y
                         float* wY, double* out3, void* stream);
 int pspde_adam_flat(int64_t n, float* theta, const float* grad, float* exp_avg, float* exp_avg_sq, double lr, double beta1,
                     double beta2, double eps, int64_t step, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
+ * Ensembles: M independent models of ONE configuration (same cfg -- problem, network geometry, K, N, dt, process --
+ * and the same problem pack `prob` and u_L2 table), trained together with one launch per phase for all of them, so that
+ * M small runs (the reference's notebooks train on K = 50 .. 256 paths: 1 .. 4 tiles, a few CTAs of the 148 SMs) fill
+ * the GPU.  Members differ in Philox key, parameters, start point(s), y0 and optimizer settings.  Member m's result is
+ * the result of the single-model entry point with key seeds[m] on its own slices: per-path outputs always bit for bit,
+ * statistics and gradient bit for bit whenever M * ceil(K_local / 64) <= #SMs (see DESIGN.md, "Ensembles", for the
+ * grid above that).  The ensemble entry points always run the FP32-FMA kernels (PSPDE_FWD_PATH / PSPDE_BWD_PATH are
+ * ignored), in-kernel Philox noise only (noise_mode INJECT is refused with -5). */
+typedef struct pspde_ensemble {
+  int32_t n_models;                 /* M >= 1                                                                          */
+  const uint64_t* seeds;            /* device, M Philox keys (cfg->seed is ignored)                                    */
+  int64_t theta_stride;             /* floats between members in theta / grad_theta, >= pspde_theta_size(cfg)          */
+  int64_t x0_stride;                /* floats between members' x0 (0 = one x0 -- a row or K_local rows -- for all)     */
+} pspde_ensemble;
+
+/* scratch bytes of pspde_ensemble_fwd / pspde_ensemble_bwd_detached for cfg and ens (0 on invalid input) */
+size_t pspde_ensemble_workspace_bytes(const pspde_cfg* cfg, const pspde_ensemble* ens);
+
+/* pspde_rollout_fwd_diag for every member in one rollout launch + one statistics launch: X_N [M][K_local][d] (nullable),
+ * Y_N / gX / Zsum [M][K_local], stats [M][4] (nullable), diag->uL2 [M][K_local] (diag nullable; the table is shared).
+ * x0: one row of d floats or (cfg->x0_per_path) K_local rows per member, member m at x0 + m * ens->x0_stride.
+ * y0: nullable, else M device floats (member m starts Y at y0[m]). */
+int pspde_ensemble_fwd(const pspde_cfg* cfg, const pspde_ensemble* ens, const float* theta, const float* prob,
+                       const float* x0, const float* y0, float* X_N, float* Y_N, float* gX, float* Zsum, double* stats,
+                       const pspde_udiag* diag, void* workspace, size_t workspace_bytes, void* stream);
+
+/* pspde_rollout_bwd_detached (FP32-FMA recompute kernel) for every member in one launch + one reduction launch:
+ * wY / wZ [M][K_local] (wZ nullable), grad_theta [M][theta_stride] (the first pspde_theta_size floats of each member
+ * are overwritten, the rest of the stride is not touched).  -6 for a network the FMA backward refuses. */
+int pspde_ensemble_bwd_detached(const pspde_cfg* cfg, const pspde_ensemble* ens, const float* theta, const float* prob,
+                                const float* x0, const float* wY, const float* wZ, float* grad_theta, void* workspace,
+                                size_t workspace_bytes, void* stream);
+
+/* pspde_lv_cotangents for n_models members in one launch: Y_N / gX / wY [M][K_local], stats [M][4], out3 [M][3]. */
+int pspde_ensemble_lv_cotangents(int32_t n_models, int K_local, double K_global, int moment, const float* Y_N,
+                                 const float* gX, const double* stats, float* wY, double* out3, void* stream);
+
+/* One member's Adam step as fp32 scalars, formed in double and rounded once (like the Python floats torch hands to its
+ * kernels; pspde_adam_flat forms the same ones).  step 0 marks a member that is not updated. */
+typedef struct pspde_adam_member {
+  float lr_over_bc1, sqrt_bc2, one_minus_beta1, beta2, one_minus_beta2, eps;   /* bc_i = 1 - beta_i^step */
+  int32_t step;
+  int32_t reserved;
+} pspde_adam_member;
+/* host function: fills *out for (lr, beta1, beta2, eps, step); step 0 gives the "skip" entry */
+int pspde_adam_member_make(double lr, double beta1, double beta2, double eps, int64_t step, pspde_adam_member* out);
+/* pspde_adam_flat for n_models members in one launch: member m updates the n floats at m * stride of theta, grad,
+ * exp_avg and exp_avg_sq with table[m] (device, n_models entries); members with table[m].step == 0 are left untouched. */
+int pspde_ensemble_adam(int32_t n_models, int64_t n, int64_t stride, float* theta, const float* grad, float* exp_avg,
+                        float* exp_avg_sq, const pspde_adam_member* table, void* stream);
 
 /* Forward + backward for detach_forward=False (solver.py:451-469 without the detach, :221): per tile of paths the
  * states X_n are checkpointed to the workspace and the discrete adjoint runs backwards in time in the same kernel.

@@ -181,11 +181,15 @@ static size_t grad_part_floats(const pspde_cfg* cfg, const Plan& pl, int s0) {
 }
 
 // FP32-FMA kernels: weight-image partials of nparts CTAs -> grad_theta (reduce_grad_image_kernel)
-static int reduce_grad_image(const Plan& pl, const RolloutParams& p, int nparts, float* grad_theta, void* stream) {
+// (ensembles: n_models members of nparts partials each, member m's gradient at grad_theta + m out_stride)
+static int reduce_grad_image(const Plan& pl, const RolloutParams& p, int nparts, float* grad_theta, void* stream,
+                             int n_models = 1, long long out_stride = 0) {
   if (!p.th_tbl) return fail(-13, "could not allocate the weight-image index table");
-  const int w4 = pl.g.w_floats >> 2, tot = pl.n_sets * w4;
-  PSPDE_LAUNCH(reduce_grad_image_kernel, (tot + 255) / 256, 256, 0, stream, p.grad_partial, nparts, pl.n_sets, w4, p.th_tbl,
-               pl.g.n_params, grad_theta);
+  const int w4 = pl.g.w_floats >> 2;
+  const long long tot = (long long)n_models * pl.n_sets * w4;
+  if (tot > 0x7fffffffLL) return fail(-6, "ensemble too large for one gradient reduction (%lld float4s)", tot);
+  PSPDE_LAUNCH(reduce_grad_image_kernel, (int)((tot + 255) / 256), 256, 0, stream, p.grad_partial, nparts, pl.n_sets, w4,
+               p.th_tbl, pl.g.n_params, grad_theta, n_models, out_stride);
   g_launches++;
   if (const char* e = pspde_peek_error()) return fail(-12, "reduce_grad launch failed: %s", e);
   return 0;
@@ -301,29 +305,105 @@ static int set_udiag(const pspde_cfg* cfg, const pspde_udiag* diag, RolloutParam
   return 0;
 }
 
+// ---- ensembles (pspde_ensemble_*): M members in one launch per phase, FP32-FMA kernels only
+struct EnsPlan {
+  Plan pl;              // pl.grid = M * grid_x: the launch
+  int grid_x;           // CTAs per member
+  size_t stats_bytes, grad_bytes;
+};
+
+// Grid policy.  While M * n_tiles <= #SMs every member gets the standalone grid (min(n_tiles, #SMs) = n_tiles, then
+// PSPDE_MAX_GRID): its CTAs run a standalone launch's tiles in the same order, so statistics and gradient are bit-equal to
+// the single-model call.  Beyond that the members share the SMs: grid_x = max(1, #SMs / M) CTAs each, so that one wave of
+// M * grid_x CTAs (one per SM: the kernels need up to 227 KB of shared memory and 128 registers a thread) covers the
+// ensemble; a member's tiles are then summed in a different grouping (results within fp32 rounding of the standalone
+// call).  PSPDE_MAX_GRID caps grid_x.
+static int make_ens_plan(const pspde_cfg* cfg, const pspde_ensemble* ens, bool bwd, EnsPlan& ep) {
+  if (!ens || ens->n_models < 1) return fail(-1, "bad ensemble descriptor (n_models >= 1)");
+  int rc = make_plan(cfg, bwd, false, ep.pl);
+  if (rc) return rc;
+  if (cfg->noise_mode != PSPDE_NOISE_PHILOX) return fail(-5, "ensembles draw their increments in the kernel (noise_mode PHILOX)");
+  if (ens->theta_stride < ep.pl.n_theta_total || ens->x0_stride < 0)
+    return fail(-1, "bad ensemble strides (theta_stride %lld < %d or x0_stride < 0)", (long long)ens->theta_stride,
+                ep.pl.n_theta_total);
+  const int M = ens->n_models, sms = pspde_sm_count();
+  int gx = ep.pl.n_tiles < sms ? ep.pl.n_tiles : sms;
+  if ((long long)M * ep.pl.n_tiles > sms) gx = sms / M > 1 ? sms / M : 1;
+  apply_max_grid(gx);
+  if ((long long)M * gx > 0x7fffffffLL) return fail(-1, "too many models for one launch (%d)", M);
+  ep.grid_x = gx;
+  ep.pl.grid = M * gx;
+  ep.stats_bytes = align256((size_t)ep.pl.grid * 4 * sizeof(double));
+  ep.grad_bytes = bwd ? align256((size_t)ep.pl.grid * ep.pl.n_img_total * sizeof(float)) : 0;
+  return 0;
+}
+
+static void set_ensemble(const pspde_ensemble* ens, const EnsPlan& ep, RolloutParams& p) {
+  p.grid_x = ep.grid_x;
+  p.theta_stride = ens->theta_stride;
+  p.x0_stride = ens->x0_stride;
+  p.seeds = reinterpret_cast<const unsigned long long*>(ens->seeds);
+}
+
 extern "C" {
 
 int pspde_abi_version(void) { return PSPDE_ABI_VERSION; }
 
 int pspde_lv_cotangents(int K_local, double K_global, int moment, const float* Y_N, const float* gX, const double* stats,
                         float* wY, double* out3, void* stream) {
-  if (K_local < 1 || !(K_global >= 1.0) || !Y_N || !gX || !stats || !wY || !out3) return fail(-1, "bad arguments");
-  PSPDE_LAUNCH(lv_cotangents_kernel, (K_local + 255) / 256, 256, 0, stream, K_local, K_global, moment, Y_N, gX, stats, wY, out3);
+  return pspde_ensemble_lv_cotangents(1, K_local, K_global, moment, Y_N, gX, stats, wY, out3, stream);
+}
+
+int pspde_ensemble_lv_cotangents(int32_t n_models, int K_local, double K_global, int moment, const float* Y_N,
+                                 const float* gX, const double* stats, float* wY, double* out3, void* stream) {
+  if (n_models < 1 || K_local < 1 || !(K_global >= 1.0) || !Y_N || !gX || !stats || !wY || !out3) return fail(-1, "bad arguments");
+  const long long blocks = (long long)n_models * ((K_local + 255) / 256);
+  if (blocks > 0x7fffffffLL) return fail(-1, "too many models for one launch");
+  PSPDE_LAUNCH(lv_cotangents_kernel, (int)blocks, 256, 0, stream, K_local, K_global, moment, Y_N, gX, stats, wY, out3);
   g_launches++;
   if (const char* e = pspde_peek_error()) return fail(-12, "lv_cotangents launch failed: %s", e);
   return 0;
 }
 
-int pspde_adam_flat(int64_t n, float* theta, const float* grad, float* exp_avg, float* exp_avg_sq, double lr, double beta1,
-                    double beta2, double eps, int64_t step, void* stream) {
-  if (n < 1 || n > 0x7fffffffLL || !theta || !grad || !exp_avg || !exp_avg_sq || step < 1) return fail(-1, "bad arguments");
-  // every scalar is formed in double and rounded once, like the Python floats torch hands to its kernels
+int pspde_adam_member_make(double lr, double beta1, double beta2, double eps, int64_t step, pspde_adam_member* out) {
+  if (!out || step < 0 || step > 0x7fffffffLL) return fail(-1, "bad arguments");
+  memset(out, 0, sizeof(*out));
+  if (step == 0) return 0;
+  // every scalar is formed in double and rounded once, like the Python floats torch hands to its kernels (on the host:
+  // the device's double pow is not correctly rounded, and one ulp of bc1 can move lr / bc1 across an fp32 rounding boundary)
   const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
-  PSPDE_LAUNCH(adam_flat_kernel, (int)((n + 255) / 256), 256, 0, stream, (int)n, theta, grad, exp_avg, exp_avg_sq,
-               (float)(lr / bc1), (float)sqrt(bc2), (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)eps);
+  out->lr_over_bc1 = (float)(lr / bc1); out->sqrt_bc2 = (float)sqrt(bc2);
+  out->one_minus_beta1 = (float)(1.0 - beta1); out->beta2 = (float)beta2; out->one_minus_beta2 = (float)(1.0 - beta2);
+  out->eps = (float)eps; out->step = (int32_t)step;
+  return 0;
+}
+
+static int launch_adam(int32_t n_models, int64_t n, int64_t stride, float* theta, const float* grad, float* exp_avg,
+                       float* exp_avg_sq, const pspde_adam_member* table, const pspde_adam_member& one, void* stream) {
+  if (n_models < 1 || n < 1 || n > 0x7fffffffLL || (n_models > 1 && stride < n) || !theta || !grad || !exp_avg || !exp_avg_sq)
+    return fail(-1, "bad arguments");
+  const long long blocks = (long long)n_models * ((n + 255) / 256);
+  if (blocks > 0x7fffffffLL) return fail(-1, "too many models for one launch");
+  PSPDE_LAUNCH(adam_flat_kernel, (int)blocks, 256, 0, stream, (int)n, (long long)stride, theta, grad, exp_avg, exp_avg_sq,
+               table, one);
   g_launches++;
   if (const char* e = pspde_peek_error()) return fail(-12, "adam_flat launch failed: %s", e);
   return 0;
+}
+
+int pspde_adam_flat(int64_t n, float* theta, const float* grad, float* exp_avg, float* exp_avg_sq, double lr, double beta1,
+                    double beta2, double eps, int64_t step, void* stream) {
+  pspde_adam_member one;
+  if (step < 1 || pspde_adam_member_make(lr, beta1, beta2, eps, step, &one)) return fail(-1, "bad arguments");
+  return launch_adam(1, n, n, theta, grad, exp_avg, exp_avg_sq, nullptr, one, stream);
+}
+
+int pspde_ensemble_adam(int32_t n_models, int64_t n, int64_t stride, float* theta, const float* grad, float* exp_avg,
+                        float* exp_avg_sq, const pspde_adam_member* table, void* stream) {
+  if (!table) return fail(-1, "bad arguments");
+  pspde_adam_member none;
+  memset(&none, 0, sizeof(none));
+  return launch_adam(n_models, n, stride, theta, grad, exp_avg, exp_avg_sq, table, none, stream);
 }
 const char* pspde_last_error(void) { return g_err; }
 uint64_t pspde_launch_count(void) { return g_launches.load(); }
@@ -422,7 +502,7 @@ int pspde_rollout_fwd_ckpt(const pspde_cfg* cfg, const float* theta, const float
   rc = launch_forward(cfg, pl, p, true, stream, &grid, workspace_bytes, keep_tiles);
   if (rc) return rc;
   if (stats) {
-    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, grid, stats);
+    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, grid, 1, stats);
     g_launches++;
     if (const char* e = pspde_peek_error()) return fail(-12, "reduce_stats launch failed: %s", e);
   }
@@ -608,7 +688,7 @@ int pspde_rollout_attached_diag(const pspde_cfg* cfg, const float* theta, const 
   rc = (pl.T == 256) ? pspde_launch_att_256(pl, p, stream) : pspde_launch_att_512(pl, p, stream);
   if (rc) return rc;
   if (stats) {
-    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, pl.grid, stats);
+    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, pl.grid, 1, stats);
     g_launches++;
   }
   return reduce_grad_image(pl, p, pl.grid, grad_theta, stream);
@@ -659,6 +739,69 @@ int64_t pspde_fma_probe_ex(int mode, int iters, float* sink, void* stream) {
   // FLOPs: 16 x 8 FMA-slots per iteration; a packed slot is 2 FMAs, the mixed mode has 4 packed + 8 scalar per 8 slots
   const int64_t fma_per_iter = mode == 0 ? 16 * 8 : mode == 1 ? 16 * 16 : 16 * (4 * 2 + 4 * 2);
   return (int64_t)sms * 1024 * (int64_t)iters * fma_per_iter * 2;
+}
+
+size_t pspde_ensemble_workspace_bytes(const pspde_cfg* cfg, const pspde_ensemble* ens) {
+  EnsPlan ep;
+  if (make_ens_plan(cfg, ens, false, ep)) return 0;
+  size_t need = ep.stats_bytes;
+  if (make_ens_plan(cfg, ens, true, ep) == 0) need = ep.stats_bytes + ep.grad_bytes;
+  return need;
+}
+
+int pspde_ensemble_fwd(const pspde_cfg* cfg, const pspde_ensemble* ens, const float* theta, const float* prob,
+                       const float* x0, const float* y0, float* X_N, float* Y_N, float* gX, float* Zsum, double* stats,
+                       const pspde_udiag* diag, void* workspace, size_t workspace_bytes, void* stream) {
+  EnsPlan ep;
+  int rc = make_ens_plan(cfg, ens, false, ep);
+  if (rc) return rc;
+  if (!theta || !prob || !x0 || !ens->seeds) return fail(-1, "theta/prob/x0/seeds must not be NULL");
+  if (!workspace || workspace_bytes < ep.stats_bytes) return fail(-7, "workspace too small (%zu < %zu)", workspace_bytes, ep.stats_bytes);
+  if (misaligned16(workspace)) return fail(-7, "workspace must be 16-byte aligned");
+  RolloutParams p;
+  fill_params(cfg, ep.pl, p);
+  set_ensemble(ens, ep, p);
+  p.theta = theta; p.prob = prob; p.x0 = x0; p.y0 = y0;
+  p.X_N = X_N; p.Y_N = Y_N; p.gX = gX; p.Zsum = Zsum;
+  if (diag && diag->mode != 0) {
+    rc = set_udiag(cfg, diag, p);
+    if (rc) return rc;
+  }
+  p.stats_partial = reinterpret_cast<double*>(workspace);
+  rc = launch_rollout<512, false, 1>(ep.pl, p, stream);
+  if (rc) return rc;
+  if (stats) {
+    PSPDE_LAUNCH(reduce_stats_kernel, (4 * ens->n_models + 255) / 256, 256, 0, stream, p.stats_partial, ep.grid_x,
+                 ens->n_models, stats);
+    g_launches++;
+    if (const char* e = pspde_peek_error()) return fail(-12, "reduce_stats launch failed: %s", e);
+  }
+  return 0;
+}
+
+int pspde_ensemble_bwd_detached(const pspde_cfg* cfg, const pspde_ensemble* ens, const float* theta, const float* prob,
+                                const float* x0, const float* wY, const float* wZ, float* grad_theta, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  EnsPlan ep;
+  int rc = make_ens_plan(cfg, ens, true, ep);
+  if (rc) return rc;
+  if (!theta || !prob || !x0 || !wY || !grad_theta || !ens->seeds)
+    return fail(-1, "theta/prob/x0/wY/grad_theta/seeds must not be NULL");
+  const size_t need = ep.stats_bytes + ep.grad_bytes;
+  if (!workspace || workspace_bytes < need) return fail(-7, "workspace too small (%zu < %zu)", workspace_bytes, need);
+  if (misaligned16(workspace)) return fail(-7, "workspace must be 16-byte aligned");
+  RolloutParams p;
+  fill_params(cfg, ep.pl, p);
+  set_ensemble(ens, ep, p);
+  p.theta = theta; p.prob = prob; p.x0 = x0; p.wY = wY; p.wZ = wZ;
+  p.grad_partial = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + ep.stats_bytes);
+  if (pspde_memset0(p.grad_partial, (size_t)ep.pl.grid * ep.pl.n_img_total * sizeof(float), stream))
+    return fail(-12, "memset of the gradient partials failed");
+  if (ep.pl.T == 256) rc = pspde_launch_bwd_256(ep.pl, p, stream);
+  else if (ep.pl.T == 512) rc = pspde_launch_bwd_512(ep.pl, p, stream);
+  else rc = fail(-13, "internal: no kernel for T=%d", ep.pl.T);
+  if (rc) return rc;
+  return reduce_grad_image(ep.pl, p, ep.grid_x, grad_theta, stream, ens->n_models, ens->theta_stride);
 }
 
 }  // extern "C"

@@ -132,7 +132,7 @@ static int diffusion_fwd_impl(const pspde_cfg* cfg, float T_end, const pspde_ell
   rc = launch_diffusion<false>(pl, p, stream);
   if (rc) return rc;
   if (stats) {
-    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, pl.grid, stats);
+    PSPDE_LAUNCH(reduce_stats_kernel, 1, 32, 0, stream, p.stats_partial, pl.grid, 1, stats);
     g_launches++;
     if (const char* e = pspde_peek_error()) return fail(-12, "reduce_stats launch failed: %s", e);
   }

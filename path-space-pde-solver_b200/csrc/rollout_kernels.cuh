@@ -12,6 +12,7 @@
 // The backward kernel recomputes the rollout (detach_forward=True: X does not depend on theta; SURVEY.md A.3),
 // so nothing of size K x N x d is ever written to HBM.
 #pragma once
+#include "../../include/pspde.h"
 #include "philox.cuh"
 #include "pspde_geom.h"
 #include "simt.h"
@@ -75,6 +76,14 @@ struct RolloutParams {
   const uint8_t* wpack;   // tensor-core rollout: shared-memory image of the six weight tiles in global memory (one bulk copy per
                           // CTA), or nullptr = every CTA stages its tiles from theta
   unsigned long long* prof;  // debug: per-phase clock64() totals of CTA 0 (16 slots) or nullptr
+  // FP32-FMA rollout_kernel, ensemble of independent models (pspde_ensemble_*): the 1-D grid is n_models consecutive groups
+  // of grid_x CTAs; CTA b serves member m = b / grid_x with the tiles b % grid_x, + grid_x, ... -- the tiles a standalone
+  // launch of grid_x CTAs gives its CTAs.  Member m reads theta + m theta_stride, x0 + m x0_stride, y0[m], wY / wZ at
+  // m K_local, Philox key seeds[m], and writes its per-path outputs at m K_local; its stats / gradient partials are rows
+  // b of stats_partial / grad_partial, i.e. a [member][cta] slice.  grid_x = 0: one model (grid_x = gridDim.x, key seed).
+  int grid_x;
+  long long theta_stride, x0_stride;
+  const unsigned long long* seeds;
 };
 
 // A trajectory stays in the batch if its D = Y_N - g(X_N) and Z_sum are finite and |D| is below the caller's blow-up bound.
@@ -419,20 +428,26 @@ __device__ __forceinline__ void bw_flush(f32x2 (&acc)[32], const NetGeom& g, con
 
 // weight-image partials of all CTAs -> theta layout: one thread per (parameter set, float4 of the image); the CTAs are summed
 // in index order (deterministic).  tbl = RolloutParams::th_tbl.  Every parameter is the image of exactly one entry.
+// Ensemble: n_models members, member m's nparts partials follow those of member m - 1 and its gradient goes to
+// out + m out_stride.
 static __global__ void reduce_grad_image_kernel(const float* __restrict__ partial, int nparts, int n_sets, int w4,
-                                                const int* __restrict__ tbl, int n_params, float* __restrict__ out) {
+                                                const int* __restrict__ tbl, int n_params, float* __restrict__ out,
+                                                int n_models, long long out_stride) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
-  if (q >= n_sets * w4) return;
-  const int set = q / w4, q4 = q - set * w4;
+  const int per = n_sets * w4;
+  if (q >= n_models * per) return;
+  const int mem = q / per, r = q - mem * per;
+  const int set = r / w4, q4 = r - set * w4;
   const int b0 = tbl[2 * q4], cs = tbl[2 * q4 + 1];
   if (b0 < 0) return;
+  partial += (size_t)mem * nparts * per * 4;
   float s[4] = {0.f, 0.f, 0.f, 0.f};
   for (int c = 0; c < nparts; ++c) {
     const float* v = partial + (((size_t)c * n_sets + set) * w4 + q4) * 4;
     s[0] += v[0]; s[1] += v[1]; s[2] += v[2]; s[3] += v[3];
   }
   const int nv = cs >> 28, st = cs & 0x0fffffff;
-  float* o = out + (size_t)set * n_params + b0;
+  float* o = out + (size_t)mem * out_stride + (size_t)set * n_params + b0;
   for (int c = 0; c < nv; ++c) o[c * st] = s[c];
 }
 
@@ -518,7 +533,7 @@ __device__ __forceinline__ void stage_noise(const RolloutParams& prm, int tile, 
 // (the activation tile must keep X_n until the weight gradient has been accumulated).
 template <int P, bool BWD>
 __device__ __forceinline__ void sde_step(const RolloutParams& prm, const SmemLayout& sl, float* smem, int tile,
-                                         int n, bool last, int warp, int lane, int nwarps) {
+                                         int n, bool last, int warp, int lane, int nwarps, unsigned long long seed) {
   const NetGeom& g = prm.g;
   const int d = prm.d, d4 = ceil4(d), ngrp = d4 >> 2;
   const float dt = prm.dt, sq = sqrtf(prm.dt);
@@ -557,7 +572,7 @@ __device__ __forceinline__ void sde_step(const RolloutParams& prm, const SmemLay
       for (int jb = gl; jb < ngrp; jb += G) {
         const int j0 = 4 * jb;
         const float4 z4 = ld4(zr + j0), x4 = ld4(xr + j0);
-        float4 e4 = philox ? philox_normal4(kglob, (unsigned)n, (unsigned)jb, prm.offset, prm.seed) : ld4(er + j0);
+        float4 e4 = philox ? philox_normal4(kglob, (unsigned)n, (unsigned)jb, prm.offset, seed) : ld4(er + j0);
         const float4 A4 = ld4(a_d + j0), B4 = ld4(b_d + j0), P4 = ld4(p_d + j0);
         const float4 K4 = ld4(kap + j0);
         const float zv[4] = {z4.x, z4.y, z4.z, z4.w}, xv[4] = {x4.x, x4.y, x4.z, x4.w};
@@ -615,7 +630,7 @@ __device__ __forceinline__ void sde_step(const RolloutParams& prm, const SmemLay
       const float* Bm = Am + d * d;
       if (philox) {   // the matvecs need the whole increment of the row: stage it first
         for (int jb = lane; jb < ngrp; jb += 32) {
-          float4 e4 = philox_normal4(kglob, (unsigned)n, (unsigned)jb, prm.offset, prm.seed);
+          float4 e4 = philox_normal4(kglob, (unsigned)n, (unsigned)jb, prm.offset, seed);
           if (4 * jb + 1 >= d) e4.y = 0.f;
           if (4 * jb + 2 >= d) e4.z = 0.f;
           if (4 * jb + 3 >= d) e4.w = 0.f;
@@ -775,17 +790,18 @@ __device__ __forceinline__ void net_backward_hidden(const RolloutParams& prm, co
   }
 }
 
+// x0, wY, wZ: the model's start points and cotangents (an ensemble member's slices of prm.x0 / prm.wY / prm.wZ)
 __device__ __forceinline__ void tile_init_state(const RolloutParams& prm, float* sAct, int tile, int P, bool bwd,
-                                                int tid, int nthr) {
+                                                int tid, int nthr, const float* x0, const float* wY, const float* wZ) {
   const NetGeom& g = prm.g;
   const int d = prm.d;
   for (int q = tid; q < P * d; q += nthr) {
     const int p = q / d, j = q - p * d, k = tile * P + p;
     float x = 0.f;
-    if (prm.x0_per_path) { if (k < prm.K_local) x = __ldg(prm.x0 + (size_t)k * d + j); }
-    else x = __ldg(prm.x0 + j);
+    if (prm.x0_per_path) { if (k < prm.K_local) x = __ldg(x0 + (size_t)k * d + j); }
+    else x = __ldg(x0 + j);
     if (bwd) {   // inert rows (zero cotangents, see sde_step) sit at the origin: finite activations whatever X_0 is
-      const bool live = k < prm.K_local && ((prm.wY && __ldg(prm.wY + k) != 0.f) || (prm.wZ && __ldg(prm.wZ + k) != 0.f));
+      const bool live = k < prm.K_local && ((wY && __ldg(wY + k) != 0.f) || (wZ && __ldg(wZ + k) != 0.f));
       if (!live) x = 0.f;
     }
     sAct[p * g.lda + j] = x;
@@ -815,12 +831,18 @@ __global__ void __launch_bounds__(T, 1) rollout_kernel(const RolloutParams prm) 
   double* sRed = reinterpret_cast<double*>(smem + sl.red);
   const bool outer = (g.time_mode == TIME_NONE);
   const bool inject = prm.noise_mode != NOISE_PHILOX;
+  // ensemble member of this CTA and the CTA's index within the member (RolloutParams::grid_x)
+  const int gx = prm.grid_x > 0 ? prm.grid_x : (int)gridDim.x;
+  const int mem = blockIdx.x / gx, cta = blockIdx.x - mem * gx;
+  const float* theta = prm.theta + (size_t)mem * prm.theta_stride;
+  const size_t mk = (size_t)mem * prm.K_local;      // the member's first per-path slot
+  const unsigned long long seed = prm.seeds ? __ldg(prm.seeds + mem) : prm.seed;
 
   // ---- one-time: clear every tile (pads must be zero), stage problem vectors and (inner) weights
   for (int q = sl.act + tid; q < sl.total; q += T) smem[q] = 0.f;
   __syncthreads();
   for (int q = tid; q < 7 * d; q += T) { const int v = q / d, j = q - v * d; smem[sl.prob + v * d4 + j] = __ldg(prm.prob + q); }
-  if (!outer) stage_weights(g, prm.theta, smem + sl.w, tid, T);
+  if (!outer) stage_weights(g, theta, smem + sl.w, tid, T);
 
   static_assert(NB == 1, "one 8x8 weight-gradient block per thread");
   f32x2 acc[32];
@@ -832,16 +854,17 @@ __global__ void __launch_bounds__(T, 1) rollout_kernel(const RolloutParams prm) 
   float* gp = BWD ? prm.grad_partial + (size_t)blockIdx.x * prm.n_img_total : nullptr;
   __syncthreads();
 
-  for (int tile = blockIdx.x; tile < prm.n_tiles; tile += gridDim.x) {
+  for (int tile = cta; tile < prm.n_tiles; tile += gx) {
     // ---- tile init (solver.py:365-376): X = X_0, Y = y0, Z_sum = 0
-    tile_init_state(prm, sAct, tile, P, BWD, tid, T);
+    tile_init_state(prm, sAct, tile, P, BWD, tid, T, prm.x0 + (size_t)mem * prm.x0_stride, prm.wY ? prm.wY + mk : nullptr,
+                    prm.wZ ? prm.wZ + mk : nullptr);
     for (int p = tid; p < P; p += T) {
       const int k = tile * P + p;
-      sY[p] = prm.y0 ? __ldg(prm.y0) : 0.f;
+      sY[p] = prm.y0 ? __ldg(prm.y0 + mem) : 0.f;
       sZs[p] = 0.f; sG[p] = 0.f; sY[6 * P + p] = 0.f; sY[7 * P + p] = 0.f;
       const bool ok = BWD && k < prm.K_local;
-      swY[p] = (ok && prm.wY) ? __ldg(prm.wY + k) : 0.f;
-      swZ[p] = (ok && prm.wZ) ? __ldg(prm.wZ + k) : 0.f;
+      swY[p] = (ok && prm.wY) ? __ldg(prm.wY + mk + k) : 0.f;
+      swZ[p] = (ok && prm.wZ) ? __ldg(prm.wZ + mk + k) : 0.f;
     }
     // (no barrier needed here: the step prologue below ends with one)
 
@@ -857,13 +880,13 @@ __global__ void __launch_bounds__(T, 1) rollout_kernel(const RolloutParams prm) 
       if (inject) stage_noise<P>(prm, tile, n, smem + sl.xi, tid, T);
       if (outer) {
         const int set = n_net < 0 ? 0 : (n_net >= prm.n_sets ? prm.n_sets - 1 : n_net);   // clamp like :352
-        stage_weights(g, prm.theta + (size_t)set * g.n_params, smem + sl.w, tid, T, prm.th_tbl);
+        stage_weights(g, theta + (size_t)set * g.n_params, smem + sl.w, tid, T, prm.th_tbl);
       }
       __syncthreads();
       pt_.mark(0);
       net_forward<P, (BWD ? 4 : 8)>(prm, sl, smem, warp, lane, NW, &pt_);
       pt_.mark(1);
-      sde_step<P, BWD>(prm, sl, smem, tile, n, n == N - 1, warp, lane, NW);
+      sde_step<P, BWD>(prm, sl, smem, tile, n, n == N - 1, warp, lane, NW, seed);
       __syncthreads();
       pt_.mark(2);
       if (BWD) {
@@ -894,11 +917,11 @@ __global__ void __launch_bounds__(T, 1) rollout_kernel(const RolloutParams prm) 
           const float Y = sY[tid], G = sG[tid], ZS = sZs[tid];
           const double D = (double)Y - (double)G;
           const bool keep = path_kept(D, ZS, prm.d_abs_max);
-          if (prm.Y_N) prm.Y_N[k] = keep ? Y : dropped_mark(Y);
-          if (prm.gX) prm.gX[k] = G;
-          if (prm.Zsum) prm.Zsum[k] = ZS;
-          if (prm.Fint) prm.Fint[k] = sY[6 * P + tid];
-          if (prm.uL2) prm.uL2[k] = sY[7 * P + tid];
+          if (prm.Y_N) prm.Y_N[mk + k] = keep ? Y : dropped_mark(Y);
+          if (prm.gX) prm.gX[mk + k] = G;
+          if (prm.Zsum) prm.Zsum[mk + k] = ZS;
+          if (prm.Fint) prm.Fint[mk + k] = sY[6 * P + tid];
+          if (prm.uL2) prm.uL2[mk + k] = sY[7 * P + tid];
           if (keep) { s0 = D; s1 = D * D; s2 = (double)ZS + (double)G; }
           else s3 = 1.0;
         }
@@ -910,7 +933,7 @@ __global__ void __launch_bounds__(T, 1) rollout_kernel(const RolloutParams prm) 
       if (prm.X_N) {
         for (int q = tid; q < P * d; q += T) {
           const int p = q / d, j = q - p * d, k = tile * P + p;
-          if (k < prm.K_local) prm.X_N[(size_t)k * d + j] = sAct[p * g.lda + j];
+          if (k < prm.K_local) prm.X_N[(mk + k) * d + j] = sAct[p * g.lda + j];
         }
       }
     } else if (!outer) {
@@ -979,7 +1002,7 @@ __global__ void __launch_bounds__(T, MINB) rollout_attached_kernel(const Rollout
   __syncthreads();
 
   for (int tile = blockIdx.x; tile < prm.n_tiles; tile += gridDim.x) {
-    tile_init_state(prm, sAct, tile, P, false, tid, T);
+    tile_init_state(prm, sAct, tile, P, false, tid, T, prm.x0, nullptr, nullptr);
     for (int p = tid; p < P; p += T) {
       const int k = tile * P + p;
       sY[p] = prm.y0 ? __ldg(prm.y0) : 0.f; sZs[p] = 0.f; sG[p] = 0.f; sY[6 * P + p] = 0.f; sY[7 * P + p] = 0.f;
@@ -1002,7 +1025,7 @@ __global__ void __launch_bounds__(T, MINB) rollout_attached_kernel(const Rollout
       if (outer) stage_weights(g, prm.theta + (size_t)n * g.n_params, smem + sl.w, tid, T, prm.th_tbl);
       __syncthreads();
       net_forward<P, 4>(prm, sl, smem, warp, lane, NW);
-      sde_step<P, false>(prm, sl, smem, tile, n, n == N - 1, warp, lane, NW);
+      sde_step<P, false>(prm, sl, smem, tile, n, n == N - 1, warp, lane, NW, prm.seed);
       __syncthreads();
     }
     // ---------------- outputs + lambda_N = w grad g(X_N)
@@ -1192,13 +1215,17 @@ __global__ void __launch_bounds__(T, MINB) rollout_attached_kernel(const Rollout
 }
 
 // ------------------------------------------------------------------------------------------------ small kernels
-// deterministic cross-CTA reductions (fixed order, fp64 accumulation)
-static __global__ void reduce_stats_kernel(const double* __restrict__ partial, int nparts, double* __restrict__ out) {
-  const int i = threadIdx.x;
-  if (i < 4) {
+// deterministic cross-CTA reductions (fixed order, fp64 accumulation): one thread per (model, statistic), the nparts
+// CTAs of a model summed in index order; model m's partials follow model m - 1's, its 4 sums go to out[4 m ..]
+static __global__ void reduce_stats_kernel(const double* __restrict__ partial, int nparts, int n_models,
+                                           double* __restrict__ out) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q < 4 * n_models) {
+    const int mem = q >> 2, i = q & 3;
+    const double* pm = partial + (size_t)mem * nparts * 4;
     double s = 0.0;
-    for (int c = 0; c < nparts; ++c) s += partial[c * 4 + i];
-    out[i] = s;
+    for (int c = 0; c < nparts; ++c) s += pm[c * 4 + i];
+    out[q] = s;
   }
 }
 
@@ -1206,12 +1233,17 @@ static __global__ void reduce_stats_kernel(const double* __restrict__ partial, i
 // forward kernel accumulated (summed over the ranks by the caller): the dozen element-wise launches of the host formulation
 // in one.  stats = [sum D, sum D^2, -, #dropped] over the kept trajectories, D = Y_N - g(X_N); a dropped trajectory carries
 // Y_N = NaN (path_kept) and gets zero weight.  out = [loss, #dropped, K_eff].
+// Ensemble: the grid is one group of ceil(K_local / blockDim.x) blocks per model; model m has Y / gX / wY at m K_local,
+// stats at 4 m and out at 3 m.
 static __global__ void lv_cotangents_kernel(int K_local, double K_global, int moment, const float* __restrict__ Y,
                                             const float* __restrict__ gX, const double* __restrict__ stats,
                                             float* __restrict__ wY, double* __restrict__ out) {
+  const int nb = (K_local + blockDim.x - 1) / blockDim.x, mem = blockIdx.x / nb;
+  const size_t mk = (size_t)mem * K_local;
+  Y += mk; gX += mk; wY += mk; stats += 4 * mem; out += 3 * mem;
   const double Ke = K_global - stats[3];
   const double mean = stats[0] / Ke;
-  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  const int k = (blockIdx.x - mem * nb) * blockDim.x + threadIdx.x;
   if (k < K_local) {
     const double D = (double)(Y[k] - gX[k]);                   // fp32 subtraction, then widened: the host formulation's order
     wY[k] = isfinite(D) ? (float)((moment ? D : D - mean) * (2.0 / Ke)) : 0.f;
@@ -1235,11 +1267,19 @@ __device__ __forceinline__ float rn_sqrt(float a) { return __fsqrt_rn(a); }
 #endif
 // One Adam step over a flat parameter buffer: the op sequence of torch.optim.Adam's single-tensor form (no weight decay,
 // no amsgrad): m = lerp(m, g, 1 - b1); v = v b2 + (1 - b2) g g; theta -= (lr / bc1) m / (sqrt(v) / sqrt(bc2) + eps).
-static __global__ void adam_flat_kernel(int n, float* __restrict__ theta, const float* __restrict__ g, float* __restrict__ m,
-                                        float* __restrict__ v, float lr_over_bc1, float sqrt_bc2, float omb1, float b2, float omb2,
-                                        float eps) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) {
+// Ensemble: the grid is one group of ceil(n / blockDim.x) blocks per model; model m updates the n floats at m stride of the
+// four buffers with the scalars tbl[m] (tbl == nullptr: one model with `one`); a model whose step is 0 is left untouched.
+static __global__ void adam_flat_kernel(int n, long long stride, float* __restrict__ theta, const float* __restrict__ g,
+                                        float* __restrict__ m, float* __restrict__ v, const pspde_adam_member* __restrict__ tbl,
+                                        pspde_adam_member one) {
+  const int nb = (n + blockDim.x - 1) / blockDim.x, mem = blockIdx.x / nb;
+  const pspde_adam_member s = tbl ? tbl[mem] : one;
+  const int i = (blockIdx.x - mem * nb) * blockDim.x + threadIdx.x;
+  if (s.step != 0 && i < n) {
+    const size_t o = (size_t)mem * stride;
+    theta += o; g += o; m += o; v += o;
+    const float lr_over_bc1 = s.lr_over_bc1, sqrt_bc2 = s.sqrt_bc2, omb1 = s.one_minus_beta1, b2 = s.beta2,
+                omb2 = s.one_minus_beta2, eps = s.eps;
     const float gi = g[i];
     const float mi = rn_add(m[i], rn_mul(rn_sub(gi, m[i]), omb1));
     const float vi = rn_add(rn_mul(v[i], b2), rn_mul(rn_mul(gi, gi), omb2));

@@ -15,7 +15,7 @@ TIME_FIRST, TIME_NONE, TIME_LAST = 0, 1, 2
 NOISE_INJECT, NOISE_PHILOX = 0, 1
 DOMAIN_SPHERE, DOMAIN_BOX, DOMAIN_ANNULUS = 1, 2, 3
 H_ZERO, H_EXP_LINEAR, H_EXP_NONLINEAR, H_EXP_NONLINEAR_SIN, H_HELMHOLTZ, H_COMMITTOR = 0, 1, 2, 3, 4, 6
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpspde.so")
@@ -47,8 +47,20 @@ class pspde_elliptic(ctypes.Structure):
                 ("h_param", ctypes.c_float * 3), ("radius_in", ctypes.c_float)]
 
 
+class pspde_ensemble(ctypes.Structure):
+    _fields_ = [("n_models", ctypes.c_int32), ("seeds", ctypes.c_void_p), ("theta_stride", ctypes.c_int64),
+                ("x0_stride", ctypes.c_int64)]
+
+
+class pspde_adam_member(ctypes.Structure):
+    _fields_ = [("lr_over_bc1", ctypes.c_float), ("sqrt_bc2", ctypes.c_float), ("one_minus_beta1", ctypes.c_float),
+                ("beta2", ctypes.c_float), ("one_minus_beta2", ctypes.c_float), ("eps", ctypes.c_float),
+                ("step", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 _P = ctypes.c_void_p
 _CFG = ctypes.POINTER(pspde_cfg)
+_ENS = ctypes.POINTER(pspde_ensemble)
 _ELL = ctypes.POINTER(pspde_elliptic)
 
 PROTOTYPES = {
@@ -90,6 +102,15 @@ PROTOTYPES = {
     "pspde_lv_cotangents": (ctypes.c_int, [ctypes.c_int, ctypes.c_double, ctypes.c_int, _P, _P, _P, _P, _P, _P]),
     "pspde_adam_flat": (ctypes.c_int, [ctypes.c_int64, _P, _P, _P, _P, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                                        ctypes.c_double, ctypes.c_int64, _P]),
+    "pspde_ensemble_workspace_bytes": (ctypes.c_size_t, [_CFG, _ENS]),
+    "pspde_ensemble_fwd": (ctypes.c_int, [_CFG, _ENS, _P, _P, _P, _P, _P, _P, _P, _P, _P, ctypes.POINTER(pspde_udiag),
+                                          _P, ctypes.c_size_t, _P]),
+    "pspde_ensemble_bwd_detached": (ctypes.c_int, [_CFG, _ENS, _P, _P, _P, _P, _P, _P, _P, ctypes.c_size_t, _P]),
+    "pspde_ensemble_lv_cotangents": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int, ctypes.c_double, ctypes.c_int, _P, _P, _P,
+                                                    _P, _P, _P]),
+    "pspde_adam_member_make": (ctypes.c_int, [ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double,
+                                              ctypes.c_int64, ctypes.POINTER(pspde_adam_member)]),
+    "pspde_ensemble_adam": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int64, ctypes.c_int64, _P, _P, _P, _P, _P, _P]),
     "pspde_fma_probe": (ctypes.c_int64, [ctypes.c_int, _P, _P]),
     "pspde_fma_probe_ex": (ctypes.c_int64, [ctypes.c_int, ctypes.c_int, _P, _P]),
 }
